@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            our arm   (one process per GPU; torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  the reference's own CPU implementation of the path
+    python bench.py ... --dump-outputs DIR                   also write the timed path's outputs of its last step to DIR/*.npy
 
 Workload (BASELINE.json configs[1]): the MDQT laser-cooling thesis run, N0 = 3500 ions, detuning = -1,
 detuningDP = +1, Om = OmDP = 1, density = 2, Ge = 0.1 -- synthetic random-start ions and random S-manifold
@@ -30,8 +31,10 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 MD_PER_STEP = 40          # sampleFreq (SU:78)
+DUMP_LIMIT_BYTES = 60 << 20  # --dump-outputs writes at most this much over all ranks (+ .npy headers): < 64 MB however MB is counted
 FLOP_PER_PAIR = 34        # SURVEY.md section 8(d)
 BYTES_PER_ION_STEP = 520  # SURVEY.md section 8(d)
 FLOP_PER_ION_STEP = 1700  # SURVEY.md section 8(d): ~1.7 kflop per no-jump 12-level ion-step (sparse H, 4 stages)
@@ -109,6 +112,22 @@ def synthetic_state(n, L, job, n_traj=1):
     return R, V, psi, tp
 
 
+def dump_outputs(out_dir, eng, suffix="", limit=DUMP_LIMIT_BYTES):
+    """What a caller of the timed path receives after its last step -- the state R, V, psi, tPart, t and the forces F of the
+    last MD step -- as float64 DIR/<name><suffix>.npy. Above `limit` bytes in all, the same seeded sample of ions is kept in
+    every run, so that two builds can still be compared array for array."""
+    s = eng.download()
+    arrays = {"R": s["R"], "V": s["V"], "psi": s["psi"], "tPart": s["tPart"], "F": eng.download_forces(), "t": np.array(s["t"])}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit:
+        keep = np.sort(np.random.default_rng(0).choice(eng.N, eng.N * limit // total, replace=False))
+        ion_axis = {"R": -1, "V": -1, "F": -1, "tPart": -1, "psi": -3}
+        arrays = {k: np.take(a, keep, axis=ion_axis[k]) if k in ion_axis else a for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + suffix + ".npy"), a)
+
+
 def pinned_like(torch, a):
     t = torch.empty(a.shape, dtype=torch.float64).pin_memory()
     v = t.numpy()
@@ -173,6 +192,8 @@ def run_ours(args):
         if w % 8 == 0:
             eng.sync()
     eng.sync()
+    # the timed steps start from the seeded inputs however many warm-up steps the clock ramp took: same arguments, same outputs
+    eng.upload(R=R, V=V, psi=psi, tPart=tp, t=0.0, substep=0)
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
@@ -187,6 +208,8 @@ def run_ours(args):
         one_step()
         ends[k].record(stream)
     eng.sync(); torch.cuda.synchronize(); barrier()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng, "" if world == 1 else "_rank%d" % rank, DUMP_LIMIT_BYTES // world)
     dev_ms = sum(s.elapsed_time(e) for s, e in zip(starts, ends))
     dev_ms = max_over_ranks(dev_ms)
     clocks = sampler.stop() if sampler else None
@@ -466,7 +489,7 @@ print(json.dumps({"kind": kind, "N": int(N), "md_steps_per_step": m, "step_s": r
 def cpu_reference_run(threads, budget_s, steps, md_max=MD_PER_STEP):
     """Run the reference's CPU path for REAL: `steps` steps of m whole MD steps each (m <= 40 sized to the budget), every MD
     step = forces() + 25 x { step(); qstep(); } (SU:1369-1378). Returns the child's record (wall seconds per step)."""
-    env = dict(os.environ, OMP_NUM_THREADS=str(threads))
+    env = dict(os.environ, OMP_NUM_THREADS=str(threads), PYTHONDONTWRITEBYTECODE="1")
     out = subprocess.run([sys.executable, "-c", _CPU_CHILD % {"root": ROOT}, str(budget_s), str(steps), str(md_max)], env=env,
                          capture_output=True, text=True, timeout=900)
     return json.loads(out.stdout.strip().splitlines()[-1])
@@ -551,7 +574,12 @@ def main():
     ap.add_argument("--large-n2", type=int, default=1000000, help="second large-N pass: BASELINE configs[4], N = 10^6 (0 = skip)")
     ap.add_argument("--no-md-family", dest="md_family", action="store_false", help="skip the MD-only / 7-level pump extras")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the state and forces after the last timed step as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none to write")
     if args.impl == "reference":
         run_reference(args)
     else:
