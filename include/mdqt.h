@@ -192,6 +192,21 @@ int mdqt_set_tags(mdqt_handle* h, const uint8_t* tags);
 int mdqt_moments_begin(mdqt_handle* h, int nslots);
 int mdqt_moments_record(mdqt_handle* h, int slot);
 int mdqt_moments_download(mdqt_handle* h, double* out, int nslots);
+/* Pressure tensor (virial stress) recorder: K_ab = sum_i v_a v_b, W_ab = sum_{i<j, 0<r<rcut} d_a d_b f(r) with d = r_i - r_j the
+ * minimum image and f(r) = (1/r + kappa) exp(-kappa r) / r^2 (so that F_i = sum_j d f), in the units of R, V and mdqt_forces (unit mass),
+ * NOT divided by the volume: the virial pressure is (tr K + tr W) / (3 L^3). Ions beyond a trajectory's count (mdqt_set_ion_counts)
+ * are left out. Single-GPU handles only (a row-decomposed handle or one with a communicator: MDQT_ESTATE).
+ * mdqt_stress_begin(nslots) allocates and zeroes a device log like mdqt_moments_begin; mdqt_stress_record(slot) writes one record
+ * there WITHOUT synchronising and leaves R, V, F, the wavefunctions, tPart, t and the step counters untouched; mdqt_stress_download
+ * copies the first nslots records as double [n_traj][12][nslots] -- series-major, each of the 12 components a contiguous series:
+ * K_xx, K_yy, K_zz, K_xy, K_xz, K_yz, W_xx, W_yy, W_zz, W_xy, W_xz, W_yz. mdqt_stress_autocorr gives the Green-Kubo shear-stress
+ * autocorrelation of the first nslots records (nslots <= 6144), acf = double [n_traj][nslots]:
+ *   C(t) = 1/(3 (nslots - t)) sum_{ab = xy, xz, yz} sum_{j < nslots - t} P_ab(j) P_ab(j + t),  P = K + W;
+ * the shear viscosity is eta = 1/(L^3 T) integral C(t) dt. */
+int mdqt_stress_begin(mdqt_handle* h, int nslots);
+int mdqt_stress_record(mdqt_handle* h, int slot);
+int mdqt_stress_download(mdqt_handle* h, double* out, int nslots);
+int mdqt_stress_autocorr(mdqt_handle* h, int nslots, double* acf);
 /* Velocity distribution of the tagged ions (bit 0 of the tags), x component: pv = double [n_traj][4001] on the bins
  * (j - 2000) * 0.0025, as recordTaggedParticleMoments() / output() of the tagging programs write it (MC408L:1069-1137, FZ408L:835-893). */
 int mdqt_vel_dist_tagged(mdqt_handle* h, double* pv);

@@ -264,6 +264,26 @@ __global__ void k_autocorr_final(const double* __restrict__ partials, int nchunk
   out[((size_t)b * 4 + p) * T + t] = s / ((double)N * (double)(T - t)) - sub;
 }
 int autocorr_chunks(int nseries) { return (nseries + kAcSeries - 1) / kAcSeries; }
+
+// Green-Kubo shear-stress autocorrelation over the pressure-tensor log [B][12][nslots] (mdqt_stress_record): the three total
+// off-diagonal series P_ab = K_ab + W_ab (ab = xy, xz, yz: entries 3..5 and 9..11) are formed into series[B][3][T], then the
+// velocity-power correlator above runs on them as 3 series of one "ion" each: its first output, divided by 3 (T - t), is
+// C(t) = 1/(3 (T - t)) sum_ab sum_{j < T - t} P_ab(j) P_ab(j + t). One chunk of series per trajectory: a fixed order.
+__global__ void k_stress_series(const double* __restrict__ log, int nslots, int T, double* __restrict__ series) {
+  const int b = blockIdx.y;
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= 3 * T) return;
+  const int q = g / T, j = g % T;
+  const double* l = log + (size_t)b * kStressPerRecord * nslots;
+  series[((size_t)b * 3 + q) * T + j] = l[(size_t)(3 + q) * nslots + j] + l[(size_t)(9 + q) * nslots + j];
+}
+int stress_autocorr_max_T() { return 48 * 1024 / (int)sizeof(double); }  // k_autocorr stages one series in shared memory
+void launch_stress_autocorr(const double* log, int nslots, int B, int T, double* series, double* partials, double* out, cudaStream_t s) {
+  k_stress_series<<<dim3((3 * T + 255) / 256, B), 256, 0, s>>>(log, nslots, T, series);
+  static_assert(3 <= kAcSeries, "the three series of a trajectory form one chunk");
+  k_autocorr<<<dim3(1, (T + 255) / 256, B), 256, (size_t)T * sizeof(double), s>>>(series, 3, T, partials);
+  k_autocorr_final<<<dim3((T + 255) / 256, 1, B), 256, 0, s>>>(partials, 1, T, 3, 0.0, 0.0, out);  // the first power only: out[b][0][t]
+}
 void launch_autocorr(const double* vstore, int N, int B, int T, double sub2, double sub4, double* partials, double* out,
                      cudaStream_t s) {
   const int nseries = 3 * N, nchunks = autocorr_chunks(nseries);

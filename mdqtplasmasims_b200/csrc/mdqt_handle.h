@@ -50,6 +50,10 @@ struct mdqt_handle {
   std::vector<GraphEntry> graphs;   // small cache keyed by nsteps
   unsigned char* tags;              // [B][N] four tag bits per ion (MD-family tagged-particle recorders) or null
   double* moments; int moments_slots;  // [slots][B][23] recorded sums (mdqt_moments_begin / _record / _download)
+  // pressure-tensor recorder (mdqt_stress_begin / _record / _download / _autocorr): the log [B][12][stress_slots], the pair pass's
+  // partial 6-vectors, and the correlator's scratch (series [B][3][T], partials [B][4][T], output [B][4][T] for T <= stress_ac_cap)
+  double *stress, *stress_partials, *stress_series, *stress_ac_partials, *stress_ac_out;
+  int stress_slots, stress_ac_cap; size_t stress_partials_cap;
   mdqt_comm* comm;                  // row-decomposed runs: NCCL communicator and exchange buffers (mdqt_comm_init), or null
 };
 

@@ -146,6 +146,14 @@ __device__ __forceinline__ double sum_partials(const double* __restrict__ src, s
 void launch_to_fixed(const double* R, long long* Rfix, size_t n, double invL, double invL_lo, cudaStream_t s);
 void launch_epot(const ForceArgs& a, double* block_partials, double* result, cudaStream_t s);  // result[B]
 int epot_partials_needed(const ForceArgs& a);
+// pressure tensor record (mdqt_force.cu): the pair pass in stress mode + K from V; out[b][12][nslots] at column `slot`
+constexpr int kStressPerRecord = 12;  // K_xx K_yy K_zz K_xy K_xz K_yz, W_xx W_yy W_zz W_xy W_xz W_yz
+void launch_stress(const ForceArgs& a, double* partials, const double* V, double* out, int nslots, int slot, cudaStream_t s);
+int stress_partials_needed(const ForceArgs& a);
+// shear-stress autocorrelation (mdqt_diag.cu): acf[b][t] = 1/(3 (T - t)) sum_{ab in xy, xz, yz} sum_{j < T - t} P_ab(j) P_ab(j + t)
+// over the first T records of the stress log [B][12][nslots]; series = [B][3][T] and partials = [B][1][4][T] scratch, out = [B][4][T]
+int stress_autocorr_max_T();
+void launch_stress_autocorr(const double* log, int nslots, int B, int T, double* series, double* partials, double* out, cudaStream_t s);
 struct QTConsts;
 void launch_substeps(const QTArgs& a, const QTConsts& C, int scheme, cudaStream_t s);
 void launch_vv_positions(const VVArgs& a, cudaStream_t s);

@@ -81,6 +81,34 @@ void write_axis_temps(const std::string& dir, const char* name, const std::vecto
   fclose(fa);
 }
 
+// --stress 1 of the md program (no counterpart in the reference): the pressure tensor of every recorded step and the Green-Kubo
+// shear-stress autocorrelation, full precision (%.17g) because they feed further integrals.
+//   stressTensor.dat    k*timeStep, K_xx K_yy K_zz K_xy K_xz K_yz, W_xx W_yy W_zz W_xy W_xz W_yz (mdqt_stress_download)
+//   stressAutoCorr.dat  tD*timeStep, C(tD), eta(tD) = trapezoid integral of C from 0 to tD / (V Tbar), V = L^3 and Tbar = the stage
+//                       mean of (K_xx + K_yy + K_zz) / (3N), the quantity temperature.dat prints
+void write_stress(mdqt_handle* h, const std::string& dir, int nsteps, int N, double L, double timeStep) {
+  std::vector<double> st((size_t)12 * nsteps), acf(nsteps);
+  CKP(mdqt_stress_download(h, st.data(), nsteps));
+  CKP(mdqt_stress_autocorr(h, nsteps, acf.data()));
+  FILE* fs = open_in(dir, "stressTensor.dat", "w");
+  double tsum = 0.0;
+  for (int k = 0; k < nsteps; k++) {
+    fprintf(fs, "%.17g", k * timeStep);
+    for (int q = 0; q < 12; q++) fprintf(fs, "\t%.17g", st[(size_t)q * nsteps + k]);
+    fprintf(fs, "\n");
+    tsum += (st[k] + st[(size_t)nsteps + k] + st[(size_t)2 * nsteps + k]) / (3.0 * N);
+  }
+  fclose(fs);
+  const double Tbar = tsum / nsteps, V = L * L * L;
+  FILE* fa = open_in(dir, "stressAutoCorr.dat", "w");
+  double integral = 0.0;
+  for (int tD = 0; tD < nsteps; tD++) {
+    if (tD > 0) integral += 0.5 * (acf[tD - 1] + acf[tD]) * timeStep;
+    fprintf(fa, "%.17g\t%.17g\t%.17g\n", tD * timeStep, acf[tD], integral / (V * Tbar));
+  }
+  fclose(fa);
+}
+
 }  // namespace
 
 // ---- MonteCarloFollowedByMDAndTempAnisotropy.cpp -----------------------------------------------------------------------------
@@ -88,9 +116,14 @@ int mdqt_program_md(int argc, char** argv) {
   OptMap opt = {{"N", "4096"}, {"Gamma", "3"}, {"kappa", "0.5"}, {"density", "0.4"}, {"timeStep", "0.005"}, {"collisionFreq", "0.25"},
                 {"preSteps", "200"}, {"recordSteps", "2500"}, {"instSteps", "2500"}, {"reequilSteps", "500"}, {"establishSteps", "-1"},
                 {"relaxSteps", "2000"}, {"tempPercentDiff", "0.15"}, {"beta", "26000"}, {"establishTime", "10"}, {"oneAxis", "0"},
-                {"pairPairStep", "0.05"}, {"seed", ""}, {"saveDirectory", "data/"}, {"device", "0"}, {"program", "md"}};
+                {"pairPairStep", "0.05"}, {"seed", ""}, {"saveDirectory", "data/"}, {"device", "0"}, {"program", "md"}, {"stress", "0"}};
   bool quiet = false;
-  if (argc < 2 || argv[1][0] == '-') { fprintf(stderr, "usage: mdqt_run --program md <job> [--N n] [--Gamma x] [--kappa x] ...\n"); return 2; }
+  if (argc < 2 || argv[1][0] == '-') {
+    fprintf(stderr, "usage: mdqt_run --program md <job> [--N n] [--Gamma x] [--kappa x] ... [--stress 0|1]\n"
+                    "       --stress 1: also record the pressure tensor at every step of the recording stage (stressTensor.dat) and its\n"
+                    "                   Green-Kubo shear-stress autocorrelation with the running viscosity integral (stressAutoCorr.dat)\n");
+    return 2;
+  }
   const unsigned job = (unsigned)atof(argv[1]);  // MD:1035
   if (!parse_opts(argc, argv, 2, opt, &quiet)) return 2;
   const int N = atoi(opt["N"].c_str());
@@ -104,6 +137,7 @@ int mdqt_program_md(int argc, char** argv) {
   const int oneAxis = atoi(opt["oneAxis"].c_str());
   const double pairPairStep = atof(opt["pairPairStep"].c_str());
   const unsigned seed = opt["seed"].empty() ? (unsigned)time(NULL) + job : (unsigned)atol(opt["seed"].c_str());
+  const bool stress = atoi(opt["stress"].c_str()) != 0;
   if (recSteps > 5000) { fprintf(stderr, "mdqt_run: recordSteps must be <= 5000\n"); return 2; }
 
   // directory tree (MD:1037-1058)
@@ -181,8 +215,10 @@ int mdqt_program_md(int argc, char** argv) {
       CKP(mdqt_set_tags(h, tags.data()));
       CKP(mdqt_moments_begin(h, recSteps));
       CKP(mdqt_vstore_begin(h, recSteps));
+      if (stress) CKP(mdqt_stress_begin(h, recSteps));
       for (int k = 0; k < recSteps; k++) {
         CKP(mdqt_moments_record(h, k));                          // recordTaggedParticleMoments(k), recordTemperature()
+        if (stress) CKP(mdqt_stress_record(h, k));               // the pressure tensor of the same state: row k of temperature.dat
         if (k % 100 == 0) { if (!quiet) printf("%d\n", k); write_gr(h, dir, k, pairPairStep, rmax); }  // MD:1097-1100
         CKP(mdqt_vv_step(h, timeStep, 0.0, sigma_v, 0, 0.0));    // MDStep(k)
         CKP(mdqt_vstore_record(h, k));                           // recordVelsForAutocorrelations(k)
@@ -214,6 +250,7 @@ int mdqt_program_md(int argc, char** argv) {
         for (int tD = 0; tD < recSteps; tD++) fprintf(fa, "%lg\t%lg\n", tD * timeStep, ac[s][tD]);
         fclose(fa);
       }
+      if (stress) write_stress(h, dir, recSteps, N, L, timeStep);
       CKP(mdqt_set_tags(h, NULL));
     }
   }

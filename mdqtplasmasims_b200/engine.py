@@ -49,7 +49,8 @@ ABI_SYMBOLS = [
     "mdqt_vstore_record", "mdqt_vstore_upload", "mdqt_autocorrelations", "mdqt_diag_partial", "mdqt_vel_dist_partial",
     "mdqt_vv_steps", "mdqt_set_ion_counts", "mdqt_set_traj_seeds", "mdqt_time_forces", "mdqt_comm_unique_id", "mdqt_comm_init", "mdqt_comm_destroy",
     "mdqt_comm_exchange_positions", "mdqt_comm_allreduce", "mdqt_populations_rows", "mdqt_download_rows", "mdqt_set_tags", "mdqt_moments_begin", "mdqt_moments_record",
-    "mdqt_moments_download", "mdqt_scale_velocities", "mdqt_vel_dist_tagged",
+    "mdqt_moments_download", "mdqt_scale_velocities", "mdqt_vel_dist_tagged", "mdqt_stress_begin", "mdqt_stress_record",
+    "mdqt_stress_download", "mdqt_stress_autocorr",
 ]
 
 _lib = None
@@ -126,6 +127,10 @@ def load_library():
     L.mdqt_moments_begin.argtypes = [vp, ctypes.c_int]
     L.mdqt_moments_record.argtypes = [vp, ctypes.c_int]
     L.mdqt_moments_download.argtypes = [vp, vp, ctypes.c_int]
+    L.mdqt_stress_begin.argtypes = [vp, ctypes.c_int]
+    L.mdqt_stress_record.argtypes = [vp, ctypes.c_int]
+    L.mdqt_stress_download.argtypes = [vp, vp, ctypes.c_int]
+    L.mdqt_stress_autocorr.argtypes = [vp, ctypes.c_int, vp]
     L.mdqt_scale_velocities.argtypes = [vp, ctypes.c_double, ctypes.c_double, ctypes.c_double]
     L.mdqt_vel_dist_tagged.argtypes = [vp, vp]
     L.mdqt_time_forces.argtypes = [vp, ctypes.c_int, c_double_p]
@@ -480,6 +485,28 @@ class Engine:
     def moments_download(self, nslots):
         out = np.empty((nslots,) + self._lead() + (23,))
         self._ck(self.lib.mdqt_moments_download(self.h, _ptr(out), nslots))
+        return out
+
+    # ---- pressure (stress) tensor recorder ------------------------------------------------------------------------------
+    def stress_begin(self, nslots):
+        """Allocate and zero a device log of ``nslots`` pressure-tensor records."""
+        self._ck(self.lib.mdqt_stress_begin(self.h, nslots))
+
+    def stress_record(self, slot):
+        """Record K_ab = sum_i v_a v_b and W_ab = sum_{i<j} d_a d_b f(r) into ``slot`` (no synchronisation; the state is untouched)."""
+        self._ck(self.lib.mdqt_stress_record(self.h, slot))
+
+    def stress_download(self, nslots):
+        """The first ``nslots`` records: [n_traj?][12][nslots] = K_xx, K_yy, K_zz, K_xy, K_xz, K_yz, W_xx, ..., W_yz."""
+        out = np.empty(self._lead() + (12, nslots))
+        self._ck(self.lib.mdqt_stress_download(self.h, _ptr(out), nslots))
+        return out
+
+    def stress_autocorr(self, nslots):
+        """Shear-stress autocorrelation C(t) = 1/(3 (T - t)) sum_{ab = xy, xz, yz} sum_j P_ab(j) P_ab(j + t) of the first ``nslots``
+        records (P = K + W): [n_traj?][nslots]."""
+        out = np.empty(self._lead() + (nslots,))
+        self._ck(self.lib.mdqt_stress_autocorr(self.h, nslots, _ptr(out)))
         return out
 
     def vel_dist_tagged(self):
