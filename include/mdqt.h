@@ -207,6 +207,28 @@ int mdqt_stress_begin(mdqt_handle* h, int nslots);
 int mdqt_stress_record(mdqt_handle* h, int slot);
 int mdqt_stress_download(mdqt_handle* h, double* out, int nslots);
 int mdqt_stress_autocorr(mdqt_handle* h, int nslots, double* acf);
+/* Heat (energy) current recorder, in the units of R, V and mdqt_forces (unit mass), with d = r_i - r_j the minimum image, r = |d|,
+ * only pairs with 0 < r < rcut, phi(r) = exp(-kappa r) / r and f(r) = (1/r + kappa) exp(-kappa r) / r^2 (so that F_i = sum_j d f).
+ * Ions beyond a trajectory's count (mdqt_set_ion_counts) are left out. Per ion phi_i = sum_{j != i} phi(r_ij) and
+ * e_i = |v_i|^2 / 2 + phi_i / 2; the energy current (Irving-Kirkwood) is J_E = sum_i e_i v_i + 1/2 sum_i sum_{j != i} d (f d.v_i).
+ * One record of a trajectory holds 15 numbers:
+ *   0-2   J_kin,a = 1/2 sum_i |v_i|^2 v_ia          9-11  P_a = sum_i v_ia (total momentum)
+ *   3-5   J_pot,a = 1/2 sum_i phi_i v_ia            12    E_kin = 1/2 sum_i |v_i|^2
+ *   6-8   J_vir,a = 1/2 sum_i sum_{j != i} d_a f (d.v_i)   13    E_pot = 1/2 sum_i phi_i (= N mdqt_epot)
+ *                                                   14    tr W = 1/2 sum_i sum_{j != i} f r^2 (= W_xx + W_yy + W_zz of mdqt_stress)
+ * Single-GPU handles only (a row-decomposed handle or one with a communicator: MDQT_ESTATE). mdqt_heat_begin(nslots) allocates and
+ * zeroes a device log; mdqt_heat_record(slot) writes one record there WITHOUT synchronising and leaves R, V, F, the wavefunctions,
+ * tPart, t and the step counters untouched; mdqt_heat_download copies the first nslots records as double [n_traj][15][nslots]
+ * (series-major). mdqt_heat_autocorr gives the Green-Kubo heat-current autocorrelation of the first nslots = T records
+ * (T <= 6144), acf = double [n_traj][T]:
+ *   J_q(j) = J_kin + J_pot + J_vir - hbar P (j),  hbar = 1/(T N_b) sum_{j < T} [E_kin + E_pot + (2 E_kin + tr W)/3](j),
+ *   C(t) = 1/(3 (T - t)) sum_{a = x, y, z} sum_{j < T - t} J_q,a(j) J_q,a(j + t);
+ * hbar P is the enthalpy current, which a non-zero (conserved) total momentum would otherwise leave as a plateau in C. The thermal
+ * conductivity is lambda = 1/(L^3 T^2) integral C(t) dt, T here the temperature. */
+int mdqt_heat_begin(mdqt_handle* h, int nslots);
+int mdqt_heat_record(mdqt_handle* h, int slot);
+int mdqt_heat_download(mdqt_handle* h, double* out, int nslots);
+int mdqt_heat_autocorr(mdqt_handle* h, int nslots, double* acf);
 /* Velocity distribution of the tagged ions (bit 0 of the tags), x component: pv = double [n_traj][4001] on the bins
  * (j - 2000) * 0.0025, as recordTaggedParticleMoments() / output() of the tagging programs write it (MC408L:1069-1137, FZ408L:835-893). */
 int mdqt_vel_dist_tagged(mdqt_handle* h, double* pv);

@@ -271,6 +271,8 @@ int mdqt_create(const mdqt_params* p, mdqt_handle** out) {
   h->tags = nullptr; h->moments = nullptr; h->moments_slots = 0;
   h->stress = h->stress_partials = h->stress_series = h->stress_ac_partials = h->stress_ac_out = nullptr;
   h->stress_slots = h->stress_ac_cap = 0; h->stress_partials_cap = 0;
+  h->heat = h->heat_partials = h->heat_series = h->heat_ac_partials = h->heat_ac_out = nullptr;
+  h->heat_slots = h->heat_ac_cap = 0; h->heat_partials_cap = 0;
   h->timing = 0; h->ev_used = 0; h->stamps = nullptr; h->stamps_cap = 0;
   for (int k = 0; k < 4; k++) { h->time_ms[k] = 0; h->time_n[k] = 0; }
   plan_force(h);
@@ -325,6 +327,7 @@ int mdqt_destroy(mdqt_handle* h) {
   if (h->tags) cudaFree(h->tags);
   if (h->moments) cudaFree(h->moments);
   for (double* b : {h->stress, h->stress_partials, h->stress_series, h->stress_ac_partials, h->stress_ac_out}) if (b) cudaFree(b);
+  for (double* b : {h->heat, h->heat_partials, h->heat_series, h->heat_ac_partials, h->heat_ac_out}) if (b) cudaFree(b);
   if (h->stamps) cudaFree(h->stamps);
   if (h->seeds) cudaFree(h->seeds);
   for (GraphEntry& g : h->graphs) cudaGraphExecDestroy(g.exec);
@@ -1269,6 +1272,83 @@ int mdqt_stress_autocorr(mdqt_handle* h, int nslots, double* acf) {
   const int T = nslots;
   launch_stress_autocorr(h->stress, h->stress_slots, h->B, T, h->stress_series, h->stress_ac_partials, h->stress_ac_out, h->stream);
   CU(cudaMemcpy2DAsync(acf, (size_t)T * 8, h->stress_ac_out, (size_t)4 * T * 8, (size_t)T * 8, h->B, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  CU(cudaGetLastError());
+  return MDQT_OK;
+}
+
+// ---- heat (energy) current recorder ----
+static int heat_handle_ok(mdqt_handle* h) {
+  if (h->nrows != h->N) return fail(MDQT_ESTATE, "mdqt_heat: a row-decomposed handle holds the sums of its own rows only");
+  if (h->comm) return fail(MDQT_ESTATE, "mdqt_heat: not available on a handle with a communicator (mdqt_comm_init)");
+  return MDQT_OK;
+}
+// the pair pass writes one 8-vector per item slot / CTA; mdqt_set_ion_counts may re-plan the chunks after mdqt_heat_begin
+static int heat_partials_fit(mdqt_handle* h) {
+  const size_t need = (size_t)std::max(1, heat_partials_needed(force_args(h)));
+  if (h->heat_partials && h->heat_partials_cap >= need) return MDQT_OK;
+  CU(cudaStreamSynchronize(h->stream));
+  if (h->heat_partials) { cudaFree(h->heat_partials); h->heat_partials = nullptr; h->heat_partials_cap = 0; }
+  CU(cudaMalloc((void**)&h->heat_partials, need * sizeof(double)));
+  h->heat_partials_cap = need;
+  return MDQT_OK;
+}
+
+int mdqt_heat_begin(mdqt_handle* h, int nslots) {
+  if (!h) return fail(MDQT_EINVAL, "null handle");
+  if (nslots < 1 || nslots > (1 << 22)) return fail(MDQT_EINVAL, "nslots outside [1, 2^22]");
+  if (int rc = heat_handle_ok(h)) return rc;
+  CU(cudaSetDevice(h->p.device));
+  CU(cudaStreamSynchronize(h->stream));
+  for (double** ptr : {&h->heat, &h->heat_series, &h->heat_ac_partials, &h->heat_ac_out}) if (*ptr) { cudaFree(*ptr); *ptr = nullptr; }
+  h->heat_slots = 0;
+  const size_t n = (size_t)h->B * kHeatPerRecord * nslots;
+  CU(cudaMalloc((void**)&h->heat, n * sizeof(double)));
+  CU(cudaMemsetAsync(h->heat, 0, n * sizeof(double), h->stream));
+  const int T = std::min(nslots, stress_autocorr_max_T());  // the same correlator as the shear stress
+  CU(cudaMalloc((void**)&h->heat_series, (size_t)h->B * 3 * T * sizeof(double)));
+  CU(cudaMalloc((void**)&h->heat_ac_partials, (size_t)h->B * 4 * T * sizeof(double)));
+  CU(cudaMalloc((void**)&h->heat_ac_out, (size_t)h->B * 4 * T * sizeof(double)));
+  if (int rc = heat_partials_fit(h)) return rc;
+  h->heat_slots = nslots; h->heat_ac_cap = T;
+  return MDQT_OK;
+}
+
+int mdqt_heat_record(mdqt_handle* h, int slot) {
+  if (!h) return fail(MDQT_EINVAL, "null handle");
+  if (!h->heat) return fail(MDQT_ESTATE, "mdqt_heat_begin not called");
+  if (slot < 0 || slot >= h->heat_slots) return fail(MDQT_EINVAL, "slot outside [0, nslots)");
+  if (int rc = heat_handle_ok(h)) return rc;
+  CU(cudaSetDevice(h->p.device));
+  if (int rc = heat_partials_fit(h)) return rc;
+  refresh_fixed(h);
+  launch_heat(force_args(h), h->heat_partials, h->V, h->heat, h->heat_slots, slot, h->stream);
+  CU(cudaGetLastError());
+  return MDQT_OK;
+}
+
+int mdqt_heat_download(mdqt_handle* h, double* out, int nslots) {
+  if (!h || !out) return fail(MDQT_EINVAL, "null argument");
+  if (!h->heat) return fail(MDQT_ESTATE, "mdqt_heat_begin not called");
+  if (nslots < 1 || nslots > h->heat_slots) return fail(MDQT_EINVAL, "nslots outside [1, slots recorded]");
+  CU(cudaSetDevice(h->p.device));
+  // [B][15][heat_slots] on the device -> [B][15][nslots] on the host
+  CU(cudaMemcpy2DAsync(out, (size_t)nslots * 8, h->heat, (size_t)h->heat_slots * 8, (size_t)nslots * 8, (size_t)h->B * kHeatPerRecord,
+                       cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  CU(cudaGetLastError());
+  return MDQT_OK;
+}
+
+int mdqt_heat_autocorr(mdqt_handle* h, int nslots, double* acf) {
+  if (!h || !acf) return fail(MDQT_EINVAL, "null argument");
+  if (!h->heat) return fail(MDQT_ESTATE, "mdqt_heat_begin not called");
+  if (nslots < 1 || nslots > h->heat_slots) return fail(MDQT_EINVAL, "nslots outside [1, slots recorded]");
+  if (nslots > h->heat_ac_cap) return fail(MDQT_EINVAL, "nslots above the correlator's limit of " + std::to_string(stress_autocorr_max_T()) + " records");
+  CU(cudaSetDevice(h->p.device));
+  const int T = nslots;
+  launch_heat_autocorr(h->heat, h->heat_slots, h->B, T, h->N, h->nb, h->heat_series, h->heat_ac_partials, h->heat_ac_out, h->stream);
+  CU(cudaMemcpy2DAsync(acf, (size_t)T * 8, h->heat_ac_out, (size_t)4 * T * 8, (size_t)T * 8, h->B, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   CU(cudaGetLastError());
   return MDQT_OK;

@@ -284,6 +284,41 @@ void launch_stress_autocorr(const double* log, int nslots, int B, int T, double*
   k_autocorr<<<dim3(1, (T + 255) / 256, B), 256, (size_t)T * sizeof(double), s>>>(series, 3, T, partials);
   k_autocorr_final<<<dim3((T + 255) / 256, 1, B), 256, 0, s>>>(partials, 1, T, 3, 0.0, 0.0, out);  // the first power only: out[b][0][t]
 }
+
+// Green-Kubo heat-current autocorrelation over the heat log [B][15][nslots] (mdqt_heat_record). One CTA per trajectory forms
+//   hbar = 1/(T N_b) sum_{j < T} [E_kin + E_pot + (2 E_kin + tr W)/3](j)   (thread-strided over the slots, then a fixed tree)
+// -- the mean enthalpy per ion, so that hbar P is the enthalpy current that the conserved momentum P carries -- and the three series
+// J_q,a(j) = J_kin,a + J_pot,a + J_vir,a - hbar P_a (j) into series[B][3][T]; the velocity-power correlator then runs on them as for
+// the shear stress.
+__global__ void __launch_bounds__(256) k_heat_series(const double* __restrict__ log, int nslots, int T, int N, const int* __restrict__ nb,
+                                                     double* __restrict__ series) {
+  __shared__ double sred[256];
+  const int b = blockIdx.x, tid = threadIdx.x;
+  const double* l = log + (size_t)b * kHeatPerRecord * nslots;
+  const double* ekin = l + (size_t)12 * nslots;
+  const double* epot = l + (size_t)13 * nslots;
+  const double* trw = l + (size_t)14 * nslots;
+  double h = 0.0;
+  for (int j = tid; j < T; j += 256) h += ekin[j] + epot[j] + (2.0 * ekin[j] + trw[j]) / 3.0;
+  sred[tid] = h;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if (tid < o) sred[tid] += sred[tid + o];
+    __syncthreads();
+  }
+  const double hbar = sred[0] / ((double)T * (double)(nb ? nb[b] : N));
+  for (int g = tid; g < 3 * T; g += 256) {
+    const int q = g / T, j = g % T;
+    series[((size_t)b * 3 + q) * T + j] = l[(size_t)q * nslots + j] + l[(size_t)(3 + q) * nslots + j] + l[(size_t)(6 + q) * nslots + j] -
+                                          hbar * l[(size_t)(9 + q) * nslots + j];
+  }
+}
+void launch_heat_autocorr(const double* log, int nslots, int B, int T, int N, const int* nb, double* series, double* partials, double* out,
+                          cudaStream_t s) {
+  k_heat_series<<<B, 256, 0, s>>>(log, nslots, T, N, nb, series);
+  k_autocorr<<<dim3(1, (T + 255) / 256, B), 256, (size_t)T * sizeof(double), s>>>(series, 3, T, partials);
+  k_autocorr_final<<<dim3((T + 255) / 256, 1, B), 256, 0, s>>>(partials, 1, T, 3, 0.0, 0.0, out);  // the first power only: out[b][0][t]
+}
 void launch_autocorr(const double* vstore, int N, int B, int T, double sub2, double sub4, double* partials, double* out,
                      cudaStream_t s) {
   const int nseries = 3 * N, nchunks = autocorr_chunks(nseries);

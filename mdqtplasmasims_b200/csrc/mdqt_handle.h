@@ -54,6 +54,9 @@ struct mdqt_handle {
   // partial 6-vectors, and the correlator's scratch (series [B][3][T], partials [B][4][T], output [B][4][T] for T <= stress_ac_cap)
   double *stress, *stress_partials, *stress_series, *stress_ac_partials, *stress_ac_out;
   int stress_slots, stress_ac_cap; size_t stress_partials_cap;
+  // heat-current recorder (mdqt_heat_*): the same layout with the log [B][15][heat_slots] and partial 8-vectors
+  double *heat, *heat_partials, *heat_series, *heat_ac_partials, *heat_ac_out;
+  int heat_slots, heat_ac_cap; size_t heat_partials_cap;
   mdqt_comm* comm;                  // row-decomposed runs: NCCL communicator and exchange buffers (mdqt_comm_init), or null
 };
 

@@ -17,7 +17,9 @@ constexpr int kMomentsPerRecord = 23; // 3 axis sums of v^2 + 4 tag sets x {coun
 struct ForceArgs {
   const double* R;   // [B][3][ld] all positions
   const long long* Rfix;  // [B][3][ld] the same positions in periodic fixed point (mdqt_fixed.cuh)
-  double* F;         // [B][3][ld] result
+  // F: [B][3][ld] result. The heat-current pair pass (kModeHeat) writes no forces and reads the velocities V [B][3][ld] in the same
+  // slot instead: a field of its own would move the kernels' second parameter and change the code of every other pair kernel
+  union { double* F; const double* V; };
   double* Fpart;     // [nsplit][B][3][ld] partial sums when nsplit > 1
   unsigned* counters;// [B][itiles] arrival counters (self-resetting)
   int N, ld, B;
@@ -154,6 +156,15 @@ int stress_partials_needed(const ForceArgs& a);
 // over the first T records of the stress log [B][12][nslots]; series = [B][3][T] and partials = [B][1][4][T] scratch, out = [B][4][T]
 int stress_autocorr_max_T();
 void launch_stress_autocorr(const double* log, int nslots, int B, int T, double* series, double* partials, double* out, cudaStream_t s);
+// heat current record (mdqt_force.cu): the pair pass in heat mode (it reads V) + the kinetic sums; out[b][15][nslots] at column `slot`
+constexpr int kHeatPerRecord = 15;  // J_kin (3), J_pot (3), J_vir (3), P (3), E_kin, E_pot, tr W
+void launch_heat(const ForceArgs& a, double* partials, const double* V, double* out, int nslots, int slot, cudaStream_t s);
+int heat_partials_needed(const ForceArgs& a);
+// heat-current autocorrelation (mdqt_diag.cu): acf[b][t] = 1/(3 (T - t)) sum_a sum_{j < T - t} J_q,a(j) J_q,a(j + t) over the first T
+// records of the heat log [B][15][nslots], J_q = J_kin + J_pot + J_vir - hbar P with hbar the mean enthalpy per ion of the T records;
+// nb = per-trajectory ion counts or null (all N); series = [B][3][T] and partials = [B][1][4][T] scratch, out = [B][4][T]
+void launch_heat_autocorr(const double* log, int nslots, int B, int T, int N, const int* nb, double* series, double* partials, double* out,
+                          cudaStream_t s);
 struct QTConsts;
 void launch_substeps(const QTArgs& a, const QTConsts& C, int scheme, cudaStream_t s);
 void launch_vv_positions(const VVArgs& a, cudaStream_t s);

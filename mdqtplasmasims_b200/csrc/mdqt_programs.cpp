@@ -109,6 +109,34 @@ void write_stress(mdqt_handle* h, const std::string& dir, int nsteps, int N, dou
   fclose(fa);
 }
 
+// --heat 1 of the md program (no counterpart in the reference): the heat current of every recorded step and the Green-Kubo
+// heat-current autocorrelation, full precision (%.17g) because they feed further integrals.
+//   heatCurrent.dat    k*timeStep, J_kin (3), J_pot (3), J_vir (3), P (3), E_kin, E_pot, tr W (mdqt_heat_download)
+//   heatAutoCorr.dat   tD*timeStep, C(tD), lambda(tD) = trapezoid integral of C from 0 to tD / (V Tbar^2), V = L^3 and Tbar = the
+//                      stage mean of 2 E_kin / (3N), the quantity temperature.dat prints
+void write_heat(mdqt_handle* h, const std::string& dir, int nsteps, int N, double L, double timeStep) {
+  std::vector<double> hc((size_t)15 * nsteps), acf(nsteps);
+  CKP(mdqt_heat_download(h, hc.data(), nsteps));
+  CKP(mdqt_heat_autocorr(h, nsteps, acf.data()));
+  FILE* fh = open_in(dir, "heatCurrent.dat", "w");
+  double tsum = 0.0;
+  for (int k = 0; k < nsteps; k++) {
+    fprintf(fh, "%.17g", k * timeStep);
+    for (int q = 0; q < 15; q++) fprintf(fh, "\t%.17g", hc[(size_t)q * nsteps + k]);
+    fprintf(fh, "\n");
+    tsum += 2.0 * hc[(size_t)12 * nsteps + k] / (3.0 * N);
+  }
+  fclose(fh);
+  const double Tbar = tsum / nsteps, V = L * L * L;
+  FILE* fa = open_in(dir, "heatAutoCorr.dat", "w");
+  double integral = 0.0;
+  for (int tD = 0; tD < nsteps; tD++) {
+    if (tD > 0) integral += 0.5 * (acf[tD - 1] + acf[tD]) * timeStep;
+    fprintf(fa, "%.17g\t%.17g\t%.17g\n", tD * timeStep, acf[tD], integral / (V * Tbar * Tbar));
+  }
+  fclose(fa);
+}
+
 }  // namespace
 
 // ---- MonteCarloFollowedByMDAndTempAnisotropy.cpp -----------------------------------------------------------------------------
@@ -116,12 +144,14 @@ int mdqt_program_md(int argc, char** argv) {
   OptMap opt = {{"N", "4096"}, {"Gamma", "3"}, {"kappa", "0.5"}, {"density", "0.4"}, {"timeStep", "0.005"}, {"collisionFreq", "0.25"},
                 {"preSteps", "200"}, {"recordSteps", "2500"}, {"instSteps", "2500"}, {"reequilSteps", "500"}, {"establishSteps", "-1"},
                 {"relaxSteps", "2000"}, {"tempPercentDiff", "0.15"}, {"beta", "26000"}, {"establishTime", "10"}, {"oneAxis", "0"},
-                {"pairPairStep", "0.05"}, {"seed", ""}, {"saveDirectory", "data/"}, {"device", "0"}, {"program", "md"}, {"stress", "0"}};
+                {"pairPairStep", "0.05"}, {"seed", ""}, {"saveDirectory", "data/"}, {"device", "0"}, {"program", "md"}, {"stress", "0"}, {"heat", "0"}};
   bool quiet = false;
   if (argc < 2 || argv[1][0] == '-') {
-    fprintf(stderr, "usage: mdqt_run --program md <job> [--N n] [--Gamma x] [--kappa x] ... [--stress 0|1]\n"
+    fprintf(stderr, "usage: mdqt_run --program md <job> [--N n] [--Gamma x] [--kappa x] ... [--stress 0|1] [--heat 0|1]\n"
                     "       --stress 1: also record the pressure tensor at every step of the recording stage (stressTensor.dat) and its\n"
-                    "                   Green-Kubo shear-stress autocorrelation with the running viscosity integral (stressAutoCorr.dat)\n");
+                    "                   Green-Kubo shear-stress autocorrelation with the running viscosity integral (stressAutoCorr.dat)\n"
+                    "       --heat 1:   also record the heat current at every step of the recording stage (heatCurrent.dat) and its\n"
+                    "                   Green-Kubo autocorrelation with the running thermal-conductivity integral (heatAutoCorr.dat)\n");
     return 2;
   }
   const unsigned job = (unsigned)atof(argv[1]);  // MD:1035
@@ -138,6 +168,7 @@ int mdqt_program_md(int argc, char** argv) {
   const double pairPairStep = atof(opt["pairPairStep"].c_str());
   const unsigned seed = opt["seed"].empty() ? (unsigned)time(NULL) + job : (unsigned)atol(opt["seed"].c_str());
   const bool stress = atoi(opt["stress"].c_str()) != 0;
+  const bool heat = atoi(opt["heat"].c_str()) != 0;
   if (recSteps > 5000) { fprintf(stderr, "mdqt_run: recordSteps must be <= 5000\n"); return 2; }
 
   // directory tree (MD:1037-1058)
@@ -216,9 +247,11 @@ int mdqt_program_md(int argc, char** argv) {
       CKP(mdqt_moments_begin(h, recSteps));
       CKP(mdqt_vstore_begin(h, recSteps));
       if (stress) CKP(mdqt_stress_begin(h, recSteps));
+      if (heat) CKP(mdqt_heat_begin(h, recSteps));
       for (int k = 0; k < recSteps; k++) {
         CKP(mdqt_moments_record(h, k));                          // recordTaggedParticleMoments(k), recordTemperature()
         if (stress) CKP(mdqt_stress_record(h, k));               // the pressure tensor of the same state: row k of temperature.dat
+        if (heat) CKP(mdqt_heat_record(h, k));                   // the heat current of the same state
         if (k % 100 == 0) { if (!quiet) printf("%d\n", k); write_gr(h, dir, k, pairPairStep, rmax); }  // MD:1097-1100
         CKP(mdqt_vv_step(h, timeStep, 0.0, sigma_v, 0, 0.0));    // MDStep(k)
         CKP(mdqt_vstore_record(h, k));                           // recordVelsForAutocorrelations(k)
@@ -251,6 +284,7 @@ int mdqt_program_md(int argc, char** argv) {
         fclose(fa);
       }
       if (stress) write_stress(h, dir, recSteps, N, L, timeStep);
+      if (heat) write_heat(h, dir, recSteps, N, L, timeStep);
       CKP(mdqt_set_tags(h, NULL));
     }
   }

@@ -50,7 +50,7 @@ ABI_SYMBOLS = [
     "mdqt_vv_steps", "mdqt_set_ion_counts", "mdqt_set_traj_seeds", "mdqt_time_forces", "mdqt_comm_unique_id", "mdqt_comm_init", "mdqt_comm_destroy",
     "mdqt_comm_exchange_positions", "mdqt_comm_allreduce", "mdqt_populations_rows", "mdqt_download_rows", "mdqt_set_tags", "mdqt_moments_begin", "mdqt_moments_record",
     "mdqt_moments_download", "mdqt_scale_velocities", "mdqt_vel_dist_tagged", "mdqt_stress_begin", "mdqt_stress_record",
-    "mdqt_stress_download", "mdqt_stress_autocorr",
+    "mdqt_stress_download", "mdqt_stress_autocorr", "mdqt_heat_begin", "mdqt_heat_record", "mdqt_heat_download", "mdqt_heat_autocorr",
 ]
 
 _lib = None
@@ -131,6 +131,10 @@ def load_library():
     L.mdqt_stress_record.argtypes = [vp, ctypes.c_int]
     L.mdqt_stress_download.argtypes = [vp, vp, ctypes.c_int]
     L.mdqt_stress_autocorr.argtypes = [vp, ctypes.c_int, vp]
+    L.mdqt_heat_begin.argtypes = [vp, ctypes.c_int]
+    L.mdqt_heat_record.argtypes = [vp, ctypes.c_int]
+    L.mdqt_heat_download.argtypes = [vp, vp, ctypes.c_int]
+    L.mdqt_heat_autocorr.argtypes = [vp, ctypes.c_int, vp]
     L.mdqt_scale_velocities.argtypes = [vp, ctypes.c_double, ctypes.c_double, ctypes.c_double]
     L.mdqt_vel_dist_tagged.argtypes = [vp, vp]
     L.mdqt_time_forces.argtypes = [vp, ctypes.c_int, c_double_p]
@@ -507,6 +511,29 @@ class Engine:
         records (P = K + W): [n_traj?][nslots]."""
         out = np.empty(self._lead() + (nslots,))
         self._ck(self.lib.mdqt_stress_autocorr(self.h, nslots, _ptr(out)))
+        return out
+
+    # ---- heat (energy) current recorder -----------------------------------------------------------------------------------
+    def heat_begin(self, nslots):
+        """Allocate and zero a device log of ``nslots`` heat-current records."""
+        self._ck(self.lib.mdqt_heat_begin(self.h, nslots))
+
+    def heat_record(self, slot):
+        """Record the heat current and its companions into ``slot`` (no synchronisation; the state is untouched)."""
+        self._ck(self.lib.mdqt_heat_record(self.h, slot))
+
+    def heat_download(self, nslots):
+        """The first ``nslots`` records: [n_traj?][15][nslots] = J_kin (3), J_pot (3), J_vir (3), P (3), E_kin, E_pot, tr W
+        (definitions: include/mdqt.h)."""
+        out = np.empty(self._lead() + (15, nslots))
+        self._ck(self.lib.mdqt_heat_download(self.h, _ptr(out), nslots))
+        return out
+
+    def heat_autocorr(self, nslots):
+        """Heat-current autocorrelation C(t) = 1/(3 (T - t)) sum_a sum_j J_q,a(j) J_q,a(j + t) of the first ``nslots`` records, with
+        J_q = J_kin + J_pot + J_vir - hbar P and hbar the records' mean enthalpy per ion: [n_traj?][nslots]."""
+        out = np.empty(self._lead() + (nslots,))
+        self._ck(self.lib.mdqt_heat_autocorr(self.h, nslots, _ptr(out)))
         return out
 
     def vel_dist_tagged(self):
