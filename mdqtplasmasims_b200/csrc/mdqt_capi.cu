@@ -467,8 +467,7 @@ int mdqt_set_ion_counts(mdqt_handle* h, const int32_t* n_ions) {
     // unequal ion counts leave ~8 % of the (trajectory, row group, chunk) slots empty, and a static walk over slots then gives the warps
     // 29-34 real items each: hand the kernel the packed list of the non-empty items (two rows per lane: the batch instantiations)
     if (h->ilist) { cudaFree(h->ilist); h->ilist = nullptr; h->icount = 0; }
-    static const bool use_list = [] { const char* e = getenv("MDQT_K1_ILIST"); return !(e && e[0] == '0'); }();  // A/B knob
-    if (n_ions && h->items && h->B > 1 && h->B < (1 << 14) && h->nsplit <= 1024 && h->N <= 64 * 256 && use_list) {
+    if (n_ions && h->items && h->B > 1 && h->B < (1 << 14) && h->nsplit <= 1024 && h->N <= 64 * 256) {
       std::vector<unsigned> list;
       list.reserve((size_t)h->B * ((h->N + 63) / 64) * h->nsplit);
       for (int b = 0; b < h->B; b++) {

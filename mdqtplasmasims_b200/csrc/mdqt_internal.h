@@ -6,10 +6,7 @@
 namespace mdqt {
 
 constexpr int kForceThreads = 128;   // threads per CTA of the pair kernels
-#ifndef MDQT_EXP_T
-#define MDQT_EXP_T 1024
-#endif
-constexpr int kExpTable = MDQT_EXP_T; // entries of the 2^(j/T) table used by the fp64 exp (128: degree-5 polynomial, 1024: degree-3)
+constexpr int kExpTable = 1024;      // entries of the 2^(j/T) table used by the fp64 exp (degree-3 polynomial)
 constexpr int kVelBins = 2001;       // KDE bins of output() (SU:120-123)
 constexpr int kTagBins = 4001;        // velocity bins of the tagged-ion distribution (MC408L:1069, FZ408L:835)
 constexpr int kMomentsPerRecord = 23; // 3 axis sums of v^2 + 4 tag sets x {count, sum v_x^1..4}
@@ -100,19 +97,13 @@ struct VVArgs {
 // their start and griddepcontrol.wait before touching data of their predecessor, so the next kernel's launch latency
 // and prologue overlap the current kernel's tail. `pdl` = launch with the programmatic-serialization attribute.
 int pdl_mode();  // MDQT_PDL: 1 = always, 0 = never, unset = -1: where the plan says the kernels' warps finish together (mdqt_capi.cu)
-bool cluster_enabled();
-// cluster_y > 0: the grid's y dimension is launched as thread-block clusters of (1, cluster_y, 1)
 template <typename... KArgs, typename A0, typename A1>
-inline cudaError_t launch_kernel(void (*kern)(KArgs...), dim3 grid, dim3 block, cudaStream_t s, bool pdl, A0 a0, A1 a1, int cluster_y = 0) {
+inline cudaError_t launch_kernel(void (*kern)(KArgs...), dim3 grid, dim3 block, cudaStream_t s, bool pdl, A0 a0, A1 a1) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = 0; cfg.stream = s;
-  cudaLaunchAttribute at[2];
+  cudaLaunchAttribute at[1];
   int n = 0;
   if (pdl) { at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[n].val.programmaticStreamSerializationAllowed = 1; n++; }
-  if (cluster_y > 0) {
-    at[n].id = cudaLaunchAttributeClusterDimension;
-    at[n].val.clusterDim.x = 1; at[n].val.clusterDim.y = (unsigned)cluster_y; at[n].val.clusterDim.z = 1; n++;
-  }
   cfg.attrs = at; cfg.numAttrs = n;
   return cudaLaunchKernelEx(&cfg, kern, a0, a1);
 }

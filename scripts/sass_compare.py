@@ -3,7 +3,8 @@
 Usage: python scripts/sass_compare.py old.so new.so
 Dumps both with `cuobjdump -sass`, strips addresses and symbol operands, and reports for every kernel of the OLD library whether
 the new one holds the same instruction sequence. Names are matched after folding a bool template argument into the int of the
-same value (`Lb0E` -> `Li0E`), so that a bool parameter widened to an int mode keeps its kernels paired."""
+same value (`Lb0E` -> `Li0E`), so that a bool parameter widened to an int mode keeps its kernels paired, and after dropping a
+trailing seventh template argument `false` of k_pairs, so that k_pairs<..., 32, false> pairs with k_pairs<..., 32>."""
 import re
 import subprocess
 import sys
@@ -27,6 +28,7 @@ def kernels(path):
 
 
 def key(name):
+    name = re.sub(r"(7k_pairsI(?:L[ib]\d+E){6})Lb0EE", r"\1E", name)
     return re.sub(r"Lb([01])E", r"Li\1E", name)
 
 

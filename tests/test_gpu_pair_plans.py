@@ -1,6 +1,6 @@
 """GPU suite: every instantiation of the all-pairs loop against a per-ion error bound.
 
-The force planner picks one of 62 instantiations of k_pairs_items / k_pairs from (n_ions, n_traj, ion counts, rcut) and the
+The force planner picks one of 58 instantiations of k_pairs_items / k_pairs from (n_ions, n_traj, ion counts, rcut) and the
 developer knobs. Each case below is one such plan, run in all four modes -- forces(), Epotential(), a stress record and a heat
 record -- in both cut-off settings: SU parameters (rcut = L/2, the HL instantiations, with one coincident pair) and MD parameters
 with rcut = 0.41 L. Every ion's force component and every record entry is compared with tests/pair_reference.py against
@@ -11,13 +11,10 @@ result by orders of magnitude more. Ions beyond a job's count sit 1e-3 a from io
 
 Each case records the kernels it launched (torch.profiler, CUDA activities, in memory), and the last test requires the union to
 be every k_pairs* symbol of the loaded library, so an instantiation added without a case here fails the suite.
-MDQT_K1_ITEMS and MDQT_FORCE_* are read per handle (set in-process); MDQT_CLUSTER is read once per process (a fresh interpreter)."""
-import json
-import os
+MDQT_K1_ITEMS and MDQT_FORCE_* are read per handle (set in-process)."""
 import re
 import shutil
 import subprocess
-import sys
 from collections import namedtuple
 
 import numpy as np
@@ -28,8 +25,6 @@ from mdqtplasmasims_b200 import Engine, md_params, su_params
 from mdqtplasmasims_b200.engine import LIB_PATH
 
 pytestmark = pytest.mark.gpu
-HERE = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(HERE)
 MODES = ("forces", "epot", "stress", "heat")
 OBSERVED = set()   # normalised k_pairs* names launched by the cases of this module
 RAN = set()
@@ -68,10 +63,7 @@ for _n, _ns in ((1001, (1, 3, 7, 1, 3, 1, 3)), (3001, (5, 2, 1, 7, 1, 3, 1))):
                                         dict(RG=128, IPT=1, JSUB=2), dict(RG=128, IPT=1, JSUB=1), dict(RG=32, JSUB=8),
                                         dict(RG=32, JSUB=4)), _ns)):
         CASES.append(case("knob_n%d_%s" % (_n, "_".join("%s%s" % kv for kv in _kn.items())), _n, env=_tiles(NSPLIT=_s, **_kn)))
-# thread-block clusters (j chunks combined through distributed shared memory): MDQT_CLUSTER is read once per process
-CLUSTER_CASES = [case("cluster_js8", 1001, env=dict(_tiles(RG=32, JSUB=8, NSPLIT=3), MDQT_CLUSTER="1"), modes=("forces",)),
-                 case("cluster_js4", 1001, env=dict(_tiles(RG=32, JSUB=4, NSPLIT=2), MDQT_CLUSTER="1"), modes=("forces",))]
-ALL_CASES = {c.name: c for c in CASES + CLUSTER_CASES}
+ALL_CASES = {c.name: c for c in CASES}
 
 
 def _params(kind, c):
@@ -115,7 +107,7 @@ def _names(prof):
 
 
 def _norm(name):
-    """'void mdqt::k_pairs<1, 8, 0, 8, true, 32, false>(...)' (or cu++filt's '(int)1, (bool)1') -> 'k_pairs<1,8,0,8,true,32,false>'."""
+    """'void mdqt::k_pairs<1, 8, 0, 8, true, 32>(...)' (or cu++filt's '(int)1, (bool)1') -> 'k_pairs<1,8,0,8,true,32>'."""
     if name.startswith("_Z"):
         name = subprocess.run(["c++filt"], input=name, capture_output=True, text=True, check=True).stdout
     m = re.search(r"(k_pairs(?:_items)?)<([^>]*)>", name)
@@ -221,35 +213,6 @@ def test_plan_against_reference(name, kind, monkeypatch):
     RAN.add((name, kind))
 
 
-_CHILD = r"""
-import json, sys
-import numpy as np
-sys.path.insert(0, sys.argv[1])
-import test_gpu_pair_plans as m
-out, plan, names = m.run_case(sys.argv[2], m.ALL_CASES[sys.argv[3]])
-np.savez(sys.argv[4] + ".npz", **out)
-json.dump({"plan": list(plan), "names": sorted(names)}, open(sys.argv[4] + ".json", "w"))
-"""
-
-
-@pytest.mark.parametrize("kind", ["su", "md"])
-@pytest.mark.parametrize("name", [c.name for c in CLUSTER_CASES])
-def test_cluster_plan_against_reference(name, kind, tmp_path):
-    c = ALL_CASES[name]
-    dst = str(tmp_path / "result")
-    r = subprocess.run([sys.executable, "-c", _CHILD, HERE, kind, name, dst], cwd=ROOT, env=dict(os.environ, **c.env),
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    meta = json.load(open(dst + ".json"))
-    names = set(meta["names"])
-    assert any(",true>" in n for n in names if n.startswith("k_pairs<")), names  # the cluster instantiation ran
-    OBSERVED.update(names)
-    out = dict(np.load(dst + ".npz"))
-    worst = check_case(kind, c, out, tuple(meta["plan"]))
-    _report(kind, c, meta["plan"], worst, names)
-    RAN.add((name, kind))
-
-
 def _library_pair_kernels():
     tool = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
     sym = subprocess.run([tool, "-symbols", LIB_PATH], capture_output=True, text=True, check=True).stdout
@@ -260,7 +223,7 @@ def _library_pair_kernels():
 
 def test_every_pair_instantiation_was_launched():
     """Runs last: the cases above must have launched every k_pairs* instantiation the library holds."""
-    expected = {(c.name, k) for c in CASES + CLUSTER_CASES for k in ("su", "md")}
+    expected = {(c.name, k) for c in CASES for k in ("su", "md")}
     assert RAN == expected, "run the whole module: cases missing %s" % sorted(expected - RAN)[:8]
     lib = _library_pair_kernels()
     missing, extra = sorted(lib - OBSERVED), sorted(OBSERVED - lib)

@@ -1,8 +1,7 @@
 """GPU suite, part 3: the opt-in kernel mappings (environment knobs read once per process) stay parity-green:
 MDQT_QT_LANES=4|2 (four / two lanes per ion in the fused substep kernel; the default picks by system size), MDQT_K1_ITEMS=0
 (the CTA-tile force kernel where the item-walking kernel is the default), MDQT_ITEMS_IPT=2 (two rows per lane in the item kernel), MDQT_GRAPH=0
-(stream launches instead of the replayed CUDA graph), MDQT_PDL=1 (programmatic dependent launch),
-MDQT_CLUSTER=1 (j chunks combined through distributed shared memory inside a thread-block cluster) and the force-kernel plan
+(stream launches instead of the replayed CUDA graph), MDQT_PDL=1 (programmatic dependent launch) and the force-kernel plan
 overrides. Each runs __graft_entry__.smoke() -- one MD step with jumps against the oracle -- plus the
 no-jump and jump-table goldens in a fresh interpreter."""
 import os
@@ -19,8 +18,7 @@ T = {"MDQT_K1_ITEMS": "0"}  # the CTA-tile force kernel (default for N > 8192) i
 
 
 @pytest.mark.parametrize("env", [{"MDQT_QT_LANES": "4"}, {"MDQT_QT_LANES": "2"}, {"MDQT_GRAPH": "0"}, {"MDQT_PDL": "1"},
-                                 {"MDQT_ITEMS_IPT": "2"}, T, dict(T, MDQT_PDL="1"), dict(T, MDQT_CLUSTER="1"),
-                                 dict(T, MDQT_CLUSTER="1", MDQT_FORCE_RG="32", MDQT_FORCE_JSUB="4", MDQT_FORCE_NSPLIT="2"),
+                                 {"MDQT_ITEMS_IPT": "2"}, T, dict(T, MDQT_PDL="1"),
                                  dict(T, MDQT_FORCE_IPT="2", MDQT_FORCE_JSUB="4"), dict(T, MDQT_FORCE_IPT="2", MDQT_FORCE_NSPLIT="3"),
                                  dict(T, MDQT_FORCE_JSUB="1", MDQT_FORCE_NSPLIT="7")])
 def test_variant_parity(env):
