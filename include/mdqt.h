@@ -229,6 +229,25 @@ int mdqt_heat_begin(mdqt_handle* h, int nslots);
 int mdqt_heat_record(mdqt_handle* h, int slot);
 int mdqt_heat_download(mdqt_handle* h, double* out, int nslots);
 int mdqt_heat_autocorr(mdqt_handle* h, int nslots, double* acf);
+/* Density and current Fourier modes (collective modes), in the units of R and V (unit mass). The caller gives K integer vectors
+ * n = nvec[q][0..2] (1 <= K <= 1024, n != 0, |n_a| < 2^20); the wave vectors are k = (2 pi / L) n. Per trajectory b and vector q:
+ *   rho_k = sum_{i < N_b} exp(i k.r_i),   j_k = sum_{i < N_b} v_i exp(i k.r_i),
+ * ions beyond a trajectory's count (mdqt_set_ion_counts) left out; the sign convention makes d rho_k / dt = i k.j_k. The phase is
+ * exact: m = n.X mod 2^64 from the periodic fixed-point positions X (units L / 2^64), k.r = pi m / 2^63 (m as a signed integer),
+ * and cos, sin come from sincospi, so the error does not grow with |n| or with how far an ion has left the box.
+ * Single-GPU handles only (a row-decomposed handle or one with a communicator: MDQT_ESTATE). mdqt_modes_begin(nvec, K, nslots)
+ * allocates and zeroes a device log (calling it again replaces the log); mdqt_modes_record(slot) writes one record there WITHOUT
+ * synchronising and leaves R, V, F, the wavefunctions, tPart, t and the step counters untouched; mdqt_modes_download copies the first
+ * nslots records as double [n_traj][K][8][nslots] (series-major): Re rho, Im rho, Re j_x, Im j_x, Re j_y, Im j_y, Re j_z, Im j_z.
+ * mdqt_modes_autocorr gives, over the first nslots = T records (T <= 6144), with khat = n / |n|, j_L = khat.j_k, j_T = j_k - khat j_L,
+ *   F(k, t)   = 1/(N_b (T - t))   sum_{s < T - t} Re[rho_k(s) rho_k*(s + t)]   (intermediate scattering function; S(k) = F(k, 0))
+ *   C_L(k, t) = 1/(N_b (T - t))   sum_{s < T - t} Re[j_L(s) j_L*(s + t)]       (longitudinal current correlation)
+ *   C_T(k, t) = 1/(2 N_b (T - t)) sum_{s < T - t} Re[j_T(s).j_T*(s + t)]       (transverse current correlation)
+ * each double [n_traj][K][T], a NULL pointer skipping that correlation. No mean is subtracted (k != 0). */
+int mdqt_modes_begin(mdqt_handle* h, const int32_t* nvec, int K, int nslots);
+int mdqt_modes_record(mdqt_handle* h, int slot);
+int mdqt_modes_download(mdqt_handle* h, double* out, int nslots);
+int mdqt_modes_autocorr(mdqt_handle* h, int nslots, double* F, double* CL, double* CT);
 /* Velocity distribution of the tagged ions (bit 0 of the tags), x component: pv = double [n_traj][4001] on the bins
  * (j - 2000) * 0.0025, as recordTaggedParticleMoments() / output() of the tagging programs write it (MC408L:1069-1137, FZ408L:835-893). */
 int mdqt_vel_dist_tagged(mdqt_handle* h, double* pv);

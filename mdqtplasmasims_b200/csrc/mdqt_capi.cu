@@ -273,6 +273,8 @@ int mdqt_create(const mdqt_params* p, mdqt_handle** out) {
   h->stress_slots = h->stress_ac_cap = 0; h->stress_partials_cap = 0;
   h->heat = h->heat_partials = h->heat_series = h->heat_ac_partials = h->heat_ac_out = nullptr;
   h->heat_slots = h->heat_ac_cap = 0; h->heat_partials_cap = 0;
+  h->modes_nvec = nullptr; h->modes = h->modes_series = h->modes_ac_partials = h->modes_ac_out = nullptr;
+  h->modes_K = h->modes_slots = h->modes_ac_cap = 0;
   h->timing = 0; h->ev_used = 0; h->stamps = nullptr; h->stamps_cap = 0;
   for (int k = 0; k < 4; k++) { h->time_ms[k] = 0; h->time_n[k] = 0; }
   plan_force(h);
@@ -328,6 +330,8 @@ int mdqt_destroy(mdqt_handle* h) {
   if (h->moments) cudaFree(h->moments);
   for (double* b : {h->stress, h->stress_partials, h->stress_series, h->stress_ac_partials, h->stress_ac_out}) if (b) cudaFree(b);
   for (double* b : {h->heat, h->heat_partials, h->heat_series, h->heat_ac_partials, h->heat_ac_out}) if (b) cudaFree(b);
+  if (h->modes_nvec) cudaFree(h->modes_nvec);
+  for (double* b : {h->modes, h->modes_series, h->modes_ac_partials, h->modes_ac_out}) if (b) cudaFree(b);
   if (h->stamps) cudaFree(h->stamps);
   if (h->seeds) cudaFree(h->seeds);
   for (GraphEntry& g : h->graphs) cudaGraphExecDestroy(g.exec);
@@ -1348,6 +1352,92 @@ int mdqt_heat_autocorr(mdqt_handle* h, int nslots, double* acf) {
   const int T = nslots;
   launch_heat_autocorr(h->heat, h->heat_slots, h->B, T, h->N, h->nb, h->heat_series, h->heat_ac_partials, h->heat_ac_out, h->stream);
   CU(cudaMemcpy2DAsync(acf, (size_t)T * 8, h->heat_ac_out, (size_t)4 * T * 8, (size_t)T * 8, h->B, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  CU(cudaGetLastError());
+  return MDQT_OK;
+}
+
+// ---- density and current Fourier mode recorder ----
+static int modes_handle_ok(mdqt_handle* h) {
+  if (h->nrows != h->N) return fail(MDQT_ESTATE, "mdqt_modes: a row-decomposed handle holds the positions of its own rows only");
+  if (h->comm) return fail(MDQT_ESTATE, "mdqt_modes: not available on a handle with a communicator (mdqt_comm_init)");
+  return MDQT_OK;
+}
+
+int mdqt_modes_begin(mdqt_handle* h, const int32_t* nvec, int K, int nslots) {
+  if (!h || !nvec) return fail(MDQT_EINVAL, "null argument");
+  if (K < 1 || K > kModesMaxK) return fail(MDQT_EINVAL, "K outside [1, " + std::to_string(kModesMaxK) + "]");
+  if (nslots < 1 || nslots > (1 << 22)) return fail(MDQT_EINVAL, "nslots outside [1, 2^22]");
+  const int Kpad = (K + kModesTile - 1) / kModesTile * kModesTile;
+  std::vector<int32_t> nv((size_t)Kpad * 3, 0);  // the tail of the last tile: zero vectors, computed and not written
+  for (int q = 0; q < K; q++) {
+    for (int a = 0; a < 3; a++) {
+      if (nvec[3 * q + a] <= -(1 << 20) || nvec[3 * q + a] >= (1 << 20))
+        return fail(MDQT_EINVAL, "wave vector " + std::to_string(q) + ": a component with |n_a| >= 2^20");
+      nv[3 * q + a] = nvec[3 * q + a];
+    }
+    if (!nv[3 * q] && !nv[3 * q + 1] && !nv[3 * q + 2]) return fail(MDQT_EINVAL, "wave vector " + std::to_string(q) + " is zero");
+  }
+  if (int rc = modes_handle_ok(h)) return rc;
+  CU(cudaSetDevice(h->p.device));
+  CU(cudaStreamSynchronize(h->stream));
+  if (h->modes_nvec) { cudaFree(h->modes_nvec); h->modes_nvec = nullptr; }
+  for (double** ptr : {&h->modes, &h->modes_series, &h->modes_ac_partials, &h->modes_ac_out}) if (*ptr) { cudaFree(*ptr); *ptr = nullptr; }
+  h->modes_K = h->modes_slots = h->modes_ac_cap = 0;
+  const size_t BK = (size_t)h->B * K, n = BK * kModesPerRecord * nslots;
+  CU(cudaMalloc((void**)&h->modes_nvec, nv.size() * sizeof(int32_t)));
+  CU(cudaMemcpyAsync(h->modes_nvec, nv.data(), nv.size() * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMalloc((void**)&h->modes, n * sizeof(double)));
+  CU(cudaMemsetAsync(h->modes, 0, n * sizeof(double), h->stream));
+  const int T = std::min(nslots, stress_autocorr_max_T());  // the same correlator as the shear stress
+  CU(cudaMalloc((void**)&h->modes_series, BK * 10 * T * sizeof(double)));
+  CU(cudaMalloc((void**)&h->modes_ac_partials, BK * 4 * T * sizeof(double)));
+  CU(cudaMalloc((void**)&h->modes_ac_out, BK * 3 * T * sizeof(double)));
+  CU(cudaStreamSynchronize(h->stream));  // nv is a host temporary
+  h->modes_K = K; h->modes_slots = nslots; h->modes_ac_cap = T;
+  return MDQT_OK;
+}
+
+int mdqt_modes_record(mdqt_handle* h, int slot) {
+  if (!h) return fail(MDQT_EINVAL, "null handle");
+  if (!h->modes) return fail(MDQT_ESTATE, "mdqt_modes_begin not called");
+  if (slot < 0 || slot >= h->modes_slots) return fail(MDQT_EINVAL, "slot outside [0, nslots)");
+  if (int rc = modes_handle_ok(h)) return rc;
+  CU(cudaSetDevice(h->p.device));
+  refresh_fixed(h);
+  launch_modes_record(h->Rfix, h->V, h->N, h->ld, h->B, h->nb, h->modes_nvec, h->modes_K, h->modes, h->modes_slots, slot, h->stream);
+  CU(cudaGetLastError());
+  return MDQT_OK;
+}
+
+int mdqt_modes_download(mdqt_handle* h, double* out, int nslots) {
+  if (!h || !out) return fail(MDQT_EINVAL, "null argument");
+  if (!h->modes) return fail(MDQT_ESTATE, "mdqt_modes_begin not called");
+  if (nslots < 1 || nslots > h->modes_slots) return fail(MDQT_EINVAL, "nslots outside [1, slots recorded]");
+  CU(cudaSetDevice(h->p.device));
+  // [B][K][8][modes_slots] on the device -> [B][K][8][nslots] on the host
+  CU(cudaMemcpy2DAsync(out, (size_t)nslots * 8, h->modes, (size_t)h->modes_slots * 8, (size_t)nslots * 8,
+                       (size_t)h->B * h->modes_K * kModesPerRecord, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  CU(cudaGetLastError());
+  return MDQT_OK;
+}
+
+int mdqt_modes_autocorr(mdqt_handle* h, int nslots, double* F, double* CL, double* CT) {
+  if (!h) return fail(MDQT_EINVAL, "null handle");
+  if (!h->modes) return fail(MDQT_ESTATE, "mdqt_modes_begin not called");
+  if (nslots < 1 || nslots > h->modes_slots) return fail(MDQT_EINVAL, "nslots outside [1, slots recorded]");
+  if (nslots > h->modes_ac_cap) return fail(MDQT_EINVAL, "nslots above the correlator's limit of " + std::to_string(stress_autocorr_max_T()) + " records");
+  CU(cudaSetDevice(h->p.device));
+  const int T = nslots;
+  const size_t n = (size_t)h->B * h->modes_K * T;
+  double* const host[3] = {F, CL, CT};
+  double* dev[3];
+  for (int c = 0; c < 3; c++) dev[c] = host[c] ? h->modes_ac_out + c * n : nullptr;
+  launch_modes_autocorr(h->modes, h->modes_slots, h->B, h->modes_K, T, h->N, h->nb, h->modes_nvec, h->modes_series, h->modes_ac_partials,
+                        dev, h->stream);
+  for (int c = 0; c < 3; c++)
+    if (host[c]) CU(cudaMemcpyAsync(host[c], dev[c], n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   CU(cudaGetLastError());
   return MDQT_OK;

@@ -319,6 +319,130 @@ void launch_heat_autocorr(const double* log, int nslots, int B, int T, int N, co
   k_autocorr<<<dim3(1, (T + 255) / 256, B), 256, (size_t)T * sizeof(double), s>>>(series, 3, T, partials);
   k_autocorr_final<<<dim3((T + 255) / 256, 1, B), 256, 0, s>>>(partials, 1, T, 3, 0.0, 0.0, out);  // the first power only: out[b][0][t]
 }
+
+// Density and current Fourier modes (mdqt_modes_record): one CTA per (tile of kModesTile vectors, trajectory). Each thread strides
+// over the trajectory's ions, loads X, Y, Z (fixed point) and v once per ion for the whole tile, and keeps 8 sums per vector. The
+// phase is integer arithmetic: m = n.X wraps modulo 2^64 exactly, so k.r = 2 pi m / 2^64 mod 2 pi with no rounding, and
+// theta = (int64) m 2^-63 in [-1, 1) goes to sincospi -- the only rounding is the int64 -> double conversion, whatever |n| and
+// however far the ion has drifted. The sums are reduced by shuffles within each warp, then warps in order: the order depends on
+// N_b and the launch shape only, so a job's record has the same bits alone, in a batch and at any capacity. Every operation is odd
+// in v, so -V gives exactly -j. nvec is [ceil(K / kModesTile) * kModesTile][3], the tail zero vectors (their sums are not written).
+constexpr int kModesThreads = 256;
+__global__ void __launch_bounds__(kModesThreads) k_modes_record(const long long* __restrict__ Rfix, const double* __restrict__ V, int Ncap,
+                                                                int ld, const int* __restrict__ nb, const int* __restrict__ nvec, int K,
+                                                                double* __restrict__ out, int nslots, int slot) {
+  __shared__ double sred[kModesThreads / 32][kModesTile * kModesPerRecord];
+  const int b = blockIdx.y, q0 = blockIdx.x * kModesTile, tid = threadIdx.x;
+  const int N = nb ? nb[b] : Ncap;
+  const unsigned long long* X = reinterpret_cast<const unsigned long long*>(Rfix) + (size_t)b * 3 * ld;
+  const unsigned long long* Y = X + ld;
+  const unsigned long long* Z = Y + ld;
+  const double* vx = V + (size_t)b * 3 * ld;
+  const double* vy = vx + ld;
+  const double* vz = vy + ld;
+  unsigned long long n[kModesTile][3];
+#pragma unroll
+  for (int q = 0; q < kModesTile; q++)
+#pragma unroll
+    for (int a = 0; a < 3; a++) n[q][a] = (unsigned long long)(long long)nvec[(q0 + q) * 3 + a];
+  double acc[kModesTile][kModesPerRecord];
+#pragma unroll
+  for (int q = 0; q < kModesTile; q++)
+#pragma unroll
+    for (int c = 0; c < kModesPerRecord; c++) acc[q][c] = 0.0;
+  for (int i = tid; i < N; i += kModesThreads) {
+    const unsigned long long x = X[i], y = Y[i], z = Z[i];
+    const double u = vx[i], v = vy[i], w = vz[i];
+#pragma unroll
+    for (int q = 0; q < kModesTile; q++) {
+      const unsigned long long m = n[q][0] * x + n[q][1] * y + n[q][2] * z;
+      double sn, cs;
+      sincospi((double)(long long)m * 0x1p-63, &sn, &cs);
+      acc[q][0] += cs; acc[q][1] += sn;
+      acc[q][2] += u * cs; acc[q][3] += u * sn;
+      acc[q][4] += v * cs; acc[q][5] += v * sn;
+      acc[q][6] += w * cs; acc[q][7] += w * sn;
+    }
+  }
+  const int lane = tid & 31, warp = tid >> 5;
+#pragma unroll
+  for (int q = 0; q < kModesTile; q++)
+#pragma unroll
+    for (int c = 0; c < kModesPerRecord; c++) {
+      double t = acc[q][c];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) t += __shfl_down_sync(0xffffffffu, t, o);
+      if (lane == 0) sred[warp][q * kModesPerRecord + c] = t;
+    }
+  __syncthreads();
+  if (tid < kModesTile * kModesPerRecord) {
+    const int q = q0 + tid / kModesPerRecord, c = tid % kModesPerRecord;
+    double t = sred[0][tid];
+#pragma unroll
+    for (int wp = 1; wp < kModesThreads / 32; wp++) t += sred[wp][tid];
+    if (q < K) out[(((size_t)b * K + q) * kModesPerRecord + c) * nslots + slot] = t;
+  }
+}
+void launch_modes_record(const long long* Rfix, const double* V, int N, int ld, int B, const int* nb, const int* nvec, int K, double* out,
+                         int nslots, int slot, cudaStream_t s) {
+  k_modes_record<<<dim3((K + kModesTile - 1) / kModesTile, B), kModesThreads, 0, s>>>(Rfix, V, N, ld, nb, nvec, K, out, nslots, slot);
+}
+
+// The three series of the mode correlations over the first T records of the mode log [B][K][8][nslots], with khat = n / |n|:
+// rho [B K][2][T] (Re, Im), j_L = khat.j [B K][2][T] (Re, Im) and j_T = j - khat j_L [B K][6][T] (Re x, Im x, Re y, ..., Im z).
+__global__ void k_modes_series(const double* __restrict__ log, int nslots, int K, int T, const int* __restrict__ nvec,
+                               double* __restrict__ rho, double* __restrict__ jl, double* __restrict__ jt) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= T) return;
+  const int q = blockIdx.y;
+  const size_t bk = (size_t)blockIdx.z * K + q;
+  const double nx = nvec[3 * q], ny = nvec[3 * q + 1], nz = nvec[3 * q + 2];
+  const double nn = sqrt(nx * nx + ny * ny + nz * nz);
+  const double kx = nx / nn, ky = ny / nn, kz = nz / nn;
+  const double* l = log + bk * kModesPerRecord * nslots + j;
+  double r[kModesPerRecord];
+#pragma unroll
+  for (int c = 0; c < kModesPerRecord; c++) r[c] = l[(size_t)c * nslots];
+  rho[(bk * 2 + 0) * T + j] = r[0];
+  rho[(bk * 2 + 1) * T + j] = r[1];
+#pragma unroll
+  for (int p = 0; p < 2; p++) {  // p = 0: real parts, 1: imaginary parts
+    const double lon = kx * r[2 + p] + ky * r[4 + p] + kz * r[6 + p];
+    jl[(bk * 2 + p) * T + j] = lon;
+    jt[(bk * 6 + 0 + p) * T + j] = r[2 + p] - kx * lon;
+    jt[(bk * 6 + 2 + p) * T + j] = r[4 + p] - ky * lon;
+    jt[(bk * 6 + 4 + p) * T + j] = r[6 + p] - kz * lon;
+  }
+}
+// out[b][q][t] = partials[b][q][0][t] / (div N_b (T - t)): the first power of k_autocorr's sums, normalised
+__global__ void k_modes_final(const double* __restrict__ partials, int K, int T, int N, const int* __restrict__ nb, double div,
+                              double* __restrict__ out) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= T) return;
+  const int b = blockIdx.z;
+  const size_t bk = (size_t)b * K + blockIdx.y;
+  out[bk * T + t] = partials[bk * 4 * T + t] / (div * (double)(nb ? nb[b] : N) * (double)(T - t));
+}
+void launch_modes_autocorr(const double* log, int nslots, int B, int K, int T, int N, const int* nb, const int* nvec, double* series,
+                           double* partials, double* const out[3], cudaStream_t s) {
+  const int BK = B * K;
+  double* const ser[3] = {series, series + (size_t)BK * 2 * T, series + (size_t)BK * 4 * T};
+  const int nser[3] = {2, 2, 6};
+  const double div[3] = {1.0, 1.0, 2.0};
+  const dim3 tiles((T + 255) / 256, K, B);
+  k_modes_series<<<tiles, 256, 0, s>>>(log, nslots, K, T, nvec, ser[0], ser[1], ser[2]);
+  static_assert(6 <= kAcSeries, "the series of one wave vector form one chunk");
+  for (int c = 0; c < 3; c++) {
+    if (!out[c]) continue;
+    for (int z0 = 0; z0 < BK; z0 += 65535) {  // grid.z holds at most 65535 (trajectory, vector) pairs
+      const int nz = min(65535, BK - z0);
+      k_autocorr<<<dim3(1, (T + 255) / 256, nz), 256, (size_t)T * sizeof(double), s>>>(ser[c] + (size_t)z0 * nser[c] * T, nser[c], T,
+                                                                                        partials + (size_t)z0 * 4 * T);
+    }
+    k_modes_final<<<tiles, 256, 0, s>>>(partials, K, T, N, nb, div[c], out[c]);
+  }
+}
+
 void launch_autocorr(const double* vstore, int N, int B, int T, double sub2, double sub4, double* partials, double* out,
                      cudaStream_t s) {
   const int nseries = 3 * N, nchunks = autocorr_chunks(nseries);

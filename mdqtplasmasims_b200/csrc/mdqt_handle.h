@@ -57,6 +57,11 @@ struct mdqt_handle {
   // heat-current recorder (mdqt_heat_*): the same layout with the log [B][15][heat_slots] and partial 8-vectors
   double *heat, *heat_partials, *heat_series, *heat_ac_partials, *heat_ac_out;
   int heat_slots, heat_ac_cap; size_t heat_partials_cap;
+  // density/current mode recorder (mdqt_modes_*): the vectors [tiles * kModesTile][3], the log [B][K][8][modes_slots], and the
+  // correlator's scratch (series [B K][10][T], partials [B K][4][T], output [3][B K][T] for T <= modes_ac_cap)
+  int* modes_nvec;
+  double *modes, *modes_series, *modes_ac_partials, *modes_ac_out;
+  int modes_K, modes_slots, modes_ac_cap;
   mdqt_comm* comm;                  // row-decomposed runs: NCCL communicator and exchange buffers (mdqt_comm_init), or null
 };
 

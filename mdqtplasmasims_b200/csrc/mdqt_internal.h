@@ -156,6 +156,17 @@ int heat_partials_needed(const ForceArgs& a);
 // nb = per-trajectory ion counts or null (all N); series = [B][3][T] and partials = [B][1][4][T] scratch, out = [B][4][T]
 void launch_heat_autocorr(const double* log, int nslots, int B, int T, int N, const int* nb, double* series, double* partials, double* out,
                           cudaStream_t s);
+// density and current Fourier modes (mdqt_diag.cu): rho_k, j_k of the K vectors nvec [ceil(K / kModesTile) * kModesTile][3] (the tail
+// zero vectors) from the fixed-point positions; out[b][q][8][nslots] at column `slot`; nb = per-trajectory ion counts or null (all N)
+constexpr int kModesPerRecord = 8;  // Re rho, Im rho, Re j_x, Im j_x, Re j_y, Im j_y, Re j_z, Im j_z
+constexpr int kModesTile = 4;       // vectors per CTA of the record kernel
+constexpr int kModesMaxK = 1024;
+void launch_modes_record(const long long* Rfix, const double* V, int N, int ld, int B, const int* nb, const int* nvec, int K, double* out,
+                         int nslots, int slot, cudaStream_t s);
+// mode correlations over the first T records of the mode log [B][K][8][nslots]: out[0] = F, out[1] = C_L, out[2] = C_T, each [B][K][T]
+// or null (skipped); series = [B K][10][T] and partials = [B K][4][T] scratch
+void launch_modes_autocorr(const double* log, int nslots, int B, int K, int T, int N, const int* nb, const int* nvec, double* series,
+                           double* partials, double* const out[3], cudaStream_t s);
 struct QTConsts;
 void launch_substeps(const QTArgs& a, const QTConsts& C, int scheme, cudaStream_t s);
 void launch_vv_positions(const VVArgs& a, cudaStream_t s);

@@ -137,6 +137,37 @@ void write_heat(mdqt_handle* h, const std::string& dir, int nsteps, int N, doubl
   fclose(fa);
 }
 
+// --modes NMAX of the md program (no counterpart in the reference): the collective modes of the axis wave vectors k = 2 pi n / L
+// along x, y and z, n = 1..NMAX (mdqt_modes_autocorr), each averaged over the three axes, full precision (%.17g):
+//   intermediateScattering.dat   tD*timeStep, F(k_n, tD) for n = 1..NMAX
+//   currentCorrL.dat             tD*timeStep, C_L(k_n, tD) for n = 1..NMAX
+//   currentCorrT.dat             tD*timeStep, C_T(k_n, tD) for n = 1..NMAX
+//   staticStructureFactor.dat    n, k_n, S(k_n) = F(k_n, 0)
+// The recorder's vector q = 3 (n - 1) + a is n along axis a.
+void write_modes(mdqt_handle* h, const std::string& dir, int nsteps, int nmax, double L, double timeStep) {
+  const size_t K = (size_t)3 * nmax;
+  std::vector<double> ac[3];
+  for (auto& a : ac) a.resize(K * nsteps);
+  CKP(mdqt_modes_autocorr(h, nsteps, ac[0].data(), ac[1].data(), ac[2].data()));
+  auto avg = [&](const std::vector<double>& a, int n, int tD) {
+    const size_t q = (size_t)3 * (n - 1);
+    return (a[q * nsteps + tD] + a[(q + 1) * nsteps + tD] + a[(q + 2) * nsteps + tD]) / 3.0;
+  };
+  static const char* names[3] = {"intermediateScattering.dat", "currentCorrL.dat", "currentCorrT.dat"};
+  for (int c = 0; c < 3; c++) {
+    FILE* f = open_in(dir, names[c], "w");
+    for (int tD = 0; tD < nsteps; tD++) {
+      fprintf(f, "%.17g", tD * timeStep);
+      for (int n = 1; n <= nmax; n++) fprintf(f, "\t%.17g", avg(ac[c], n, tD));
+      fprintf(f, "\n");
+    }
+    fclose(f);
+  }
+  FILE* fs = open_in(dir, "staticStructureFactor.dat", "w");
+  for (int n = 1; n <= nmax; n++) fprintf(fs, "%d\t%.17g\t%.17g\n", n, 2 * M_PI * n / L, avg(ac[0], n, 0));
+  fclose(fs);
+}
+
 }  // namespace
 
 // ---- MonteCarloFollowedByMDAndTempAnisotropy.cpp -----------------------------------------------------------------------------
@@ -144,14 +175,19 @@ int mdqt_program_md(int argc, char** argv) {
   OptMap opt = {{"N", "4096"}, {"Gamma", "3"}, {"kappa", "0.5"}, {"density", "0.4"}, {"timeStep", "0.005"}, {"collisionFreq", "0.25"},
                 {"preSteps", "200"}, {"recordSteps", "2500"}, {"instSteps", "2500"}, {"reequilSteps", "500"}, {"establishSteps", "-1"},
                 {"relaxSteps", "2000"}, {"tempPercentDiff", "0.15"}, {"beta", "26000"}, {"establishTime", "10"}, {"oneAxis", "0"},
-                {"pairPairStep", "0.05"}, {"seed", ""}, {"saveDirectory", "data/"}, {"device", "0"}, {"program", "md"}, {"stress", "0"}, {"heat", "0"}};
+                {"pairPairStep", "0.05"}, {"seed", ""}, {"saveDirectory", "data/"}, {"device", "0"}, {"program", "md"}, {"stress", "0"}, {"heat", "0"},
+                {"modes", "0"}};
   bool quiet = false;
   if (argc < 2 || argv[1][0] == '-') {
-    fprintf(stderr, "usage: mdqt_run --program md <job> [--N n] [--Gamma x] [--kappa x] ... [--stress 0|1] [--heat 0|1]\n"
+    fprintf(stderr, "usage: mdqt_run --program md <job> [--N n] [--Gamma x] [--kappa x] ... [--stress 0|1] [--heat 0|1] [--modes NMAX]\n"
                     "       --stress 1: also record the pressure tensor at every step of the recording stage (stressTensor.dat) and its\n"
                     "                   Green-Kubo shear-stress autocorrelation with the running viscosity integral (stressAutoCorr.dat)\n"
                     "       --heat 1:   also record the heat current at every step of the recording stage (heatCurrent.dat) and its\n"
-                    "                   Green-Kubo autocorrelation with the running thermal-conductivity integral (heatAutoCorr.dat)\n");
+                    "                   Green-Kubo autocorrelation with the running thermal-conductivity integral (heatAutoCorr.dat)\n"
+                    "       --modes NMAX: also record the density and current Fourier modes of k = 2 pi n / L along x, y and z,\n"
+                    "                   n = 1..NMAX (at most 341), at every step of the recording stage; write the intermediate scattering\n"
+                    "                   function and the longitudinal and transverse current correlations, axis-averaged\n"
+                    "                   (intermediateScattering.dat, currentCorrL.dat, currentCorrT.dat), and S(k) (staticStructureFactor.dat)\n");
     return 2;
   }
   const unsigned job = (unsigned)atof(argv[1]);  // MD:1035
@@ -169,6 +205,8 @@ int mdqt_program_md(int argc, char** argv) {
   const unsigned seed = opt["seed"].empty() ? (unsigned)time(NULL) + job : (unsigned)atol(opt["seed"].c_str());
   const bool stress = atoi(opt["stress"].c_str()) != 0;
   const bool heat = atoi(opt["heat"].c_str()) != 0;
+  const int modes = atoi(opt["modes"].c_str());
+  if (modes < 0 || 3 * modes > 1024) { fprintf(stderr, "mdqt_run: modes must be in [0, 341]\n"); return 2; }
   if (recSteps > 5000) { fprintf(stderr, "mdqt_run: recordSteps must be <= 5000\n"); return 2; }
 
   // directory tree (MD:1037-1058)
@@ -248,10 +286,14 @@ int mdqt_program_md(int argc, char** argv) {
       CKP(mdqt_vstore_begin(h, recSteps));
       if (stress) CKP(mdqt_stress_begin(h, recSteps));
       if (heat) CKP(mdqt_heat_begin(h, recSteps));
+      std::vector<int32_t> nvec((size_t)9 * modes, 0);  // the axis vectors: q = 3 (n - 1) + a is n along axis a
+      for (int q = 0; q < 3 * modes; q++) nvec[(size_t)3 * q + q % 3] = q / 3 + 1;
+      if (modes) CKP(mdqt_modes_begin(h, nvec.data(), 3 * modes, recSteps));
       for (int k = 0; k < recSteps; k++) {
         CKP(mdqt_moments_record(h, k));                          // recordTaggedParticleMoments(k), recordTemperature()
         if (stress) CKP(mdqt_stress_record(h, k));               // the pressure tensor of the same state: row k of temperature.dat
         if (heat) CKP(mdqt_heat_record(h, k));                   // the heat current of the same state
+        if (modes) CKP(mdqt_modes_record(h, k));                 // rho_k and j_k of the same state
         if (k % 100 == 0) { if (!quiet) printf("%d\n", k); write_gr(h, dir, k, pairPairStep, rmax); }  // MD:1097-1100
         CKP(mdqt_vv_step(h, timeStep, 0.0, sigma_v, 0, 0.0));    // MDStep(k)
         CKP(mdqt_vstore_record(h, k));                           // recordVelsForAutocorrelations(k)
@@ -285,6 +327,7 @@ int mdqt_program_md(int argc, char** argv) {
       }
       if (stress) write_stress(h, dir, recSteps, N, L, timeStep);
       if (heat) write_heat(h, dir, recSteps, N, L, timeStep);
+      if (modes) write_modes(h, dir, recSteps, modes, L, timeStep);
       CKP(mdqt_set_tags(h, NULL));
     }
   }

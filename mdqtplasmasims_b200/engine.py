@@ -51,6 +51,7 @@ ABI_SYMBOLS = [
     "mdqt_comm_exchange_positions", "mdqt_comm_allreduce", "mdqt_populations_rows", "mdqt_download_rows", "mdqt_set_tags", "mdqt_moments_begin", "mdqt_moments_record",
     "mdqt_moments_download", "mdqt_scale_velocities", "mdqt_vel_dist_tagged", "mdqt_stress_begin", "mdqt_stress_record",
     "mdqt_stress_download", "mdqt_stress_autocorr", "mdqt_heat_begin", "mdqt_heat_record", "mdqt_heat_download", "mdqt_heat_autocorr",
+    "mdqt_modes_begin", "mdqt_modes_record", "mdqt_modes_download", "mdqt_modes_autocorr",
 ]
 
 _lib = None
@@ -135,6 +136,10 @@ def load_library():
     L.mdqt_heat_record.argtypes = [vp, ctypes.c_int]
     L.mdqt_heat_download.argtypes = [vp, vp, ctypes.c_int]
     L.mdqt_heat_autocorr.argtypes = [vp, ctypes.c_int, vp]
+    L.mdqt_modes_begin.argtypes = [vp, vp, ctypes.c_int, ctypes.c_int]
+    L.mdqt_modes_record.argtypes = [vp, ctypes.c_int]
+    L.mdqt_modes_download.argtypes = [vp, vp, ctypes.c_int]
+    L.mdqt_modes_autocorr.argtypes = [vp, ctypes.c_int, vp, vp, vp]
     L.mdqt_scale_velocities.argtypes = [vp, ctypes.c_double, ctypes.c_double, ctypes.c_double]
     L.mdqt_vel_dist_tagged.argtypes = [vp, vp]
     L.mdqt_time_forces.argtypes = [vp, ctypes.c_int, c_double_p]
@@ -190,6 +195,12 @@ def philox_uniforms(seed, traj, n_ions, substep):
     return u
 
 
+def axis_wavevectors(nmax):
+    """The 3 nmax integer vectors (n,0,0), (0,n,0), (0,0,n) for n = 1..nmax, in that order: int32 [3 nmax][3], so that a result over
+    them reshaped to [nmax][3] averages over the three axes along its second index."""
+    return np.concatenate([n * np.eye(3, dtype=np.int32) for n in range(1, nmax + 1)]).reshape(3 * nmax, 3)
+
+
 def _ptr(a):
     return None if a is None else ctypes.c_void_p(a.ctypes.data)
 
@@ -219,6 +230,7 @@ class Engine:
             raise MDQTError("mdqt_create failed (%d): %s" % (rc, self.lib.mdqt_last_error().decode()))
         self.h = h
         self.N, self.B, self.S = params.n_ions, params.n_traj, params.scheme
+        self._modes_K = 0  # wave vectors of the mode log (modes_begin)
 
     def close(self):
         if getattr(self, "h", None):
@@ -535,6 +547,34 @@ class Engine:
         out = np.empty(self._lead() + (nslots,))
         self._ck(self.lib.mdqt_heat_autocorr(self.h, nslots, _ptr(out)))
         return out
+
+    # ---- density and current Fourier modes ----------------------------------------------------------------------------------
+    def modes_begin(self, nvec, nslots):
+        """Allocate and zero a device log of ``nslots`` records of rho_k and j_k for the integer vectors ``nvec`` [K][3]
+        (k = 2 pi n / L; 1 <= K <= 1024, n != 0, |n_a| < 2^20)."""
+        nv = np.ascontiguousarray(nvec, dtype=np.int32)
+        if nv.ndim != 2 or nv.shape[1] != 3:
+            raise MDQTError("nvec has shape %s, expected [K][3]" % (nv.shape,))
+        self._ck(self.lib.mdqt_modes_begin(self.h, _ptr(nv), nv.shape[0], nslots))
+        self._modes_K = nv.shape[0]
+
+    def modes_record(self, slot):
+        """Record rho_k and j_k of every vector into ``slot`` (no synchronisation; the state is untouched)."""
+        self._ck(self.lib.mdqt_modes_record(self.h, slot))
+
+    def modes_download(self, nslots):
+        """The first ``nslots`` records: [n_traj?][K][8][nslots] = Re rho, Im rho, Re j_x, Im j_x, Re j_y, Im j_y, Re j_z, Im j_z
+        (definitions: include/mdqt.h)."""
+        out = np.empty(self._lead() + (self._modes_K, 8, nslots))
+        self._ck(self.lib.mdqt_modes_download(self.h, _ptr(out), nslots))
+        return out
+
+    def modes_autocorr(self, nslots):
+        """(F, C_L, C_T) of the first ``nslots`` records, each [n_traj?][K][nslots]: the intermediate scattering function and the
+        longitudinal and transverse current correlations (definitions: include/mdqt.h); S(k) = F[..., 0]."""
+        out = [np.empty(self._lead() + (self._modes_K, nslots)) for _ in range(3)]
+        self._ck(self.lib.mdqt_modes_autocorr(self.h, nslots, *(_ptr(o) for o in out)))
+        return tuple(out)
 
     def vel_dist_tagged(self):
         p = np.empty(self._lead() + (4001,))
