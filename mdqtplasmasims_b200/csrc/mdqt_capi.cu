@@ -117,26 +117,30 @@ int mdqt_params_ts(mdqt_params* p, int n_ions, double detuning, double Om) {
 
 // j-range decomposition: a function of (N, B) only, so that every rank of a row-decomposed run sums the same
 // j-chunks in the same order (bitwise identical forces for any GPU count).
-// Item-walking kernel (k_pairs_items): chunk length for `np` ions, chosen for ONE trajectory on the chip's 148 x 2 x 8
-// resident warps -- the latency-critical case; a batch walks B times as many equal items whatever the choice. A function of
-// np alone (a trajectory's own ion count -- n_ions, or its entry in mdqt_set_ion_counts -- or the nominal mdqt_params.plan_n): not of
-// the batch size, the row range or the environment.
-static int plan_items_jlen(int np) {
-  const long long W = 148LL * 2 * 8;
-  const long long G = (np + 31) / 32;
-  double best = 1e300;
-  int best_jl = 8;
-  for (int jl = 8; jl <= 256; jl += 8) {  // kItemMaxJ
-    const long long nch = (np + jl - 1) / jl;
-    const long long rounds = (G * nch + W - 1) / W;
-    // per item: jl pair iterations + ~14 iterations' worth of tile wait, partial store, fence and arrival; the last warp of
-    // a group fetches the partials in batches of 12 (one L2 round trip ~ 6 iterations each)
-    const double cost = (double)rounds * (jl + 14) + (nch > 1 ? 6.0 * ((nch + 11) / 12) : 0.0);
-    if (cost < best) { best = cost; best_jl = jl; }
-  }
-  return best_jl;
-}
 constexpr int kItemsMaxN = 8192;  // beyond this the partial-sum buffer (chunks x 3 x N) grows and CTA tiles win anyway
+
+// The tile list of the pair-once force kernel, b << 16 | I << 8 | J for the tiles I <= J < ceil(N_b / 64) of every trajectory b
+// (its own ion count: n_ions, or its entry in mdqt_set_ion_counts) that touch the handle's rows -- a row-decomposed handle runs every
+// tile whose row or column block overlaps its rows and stores its own rows' partials only, so its forces have the whole system's
+// bits. Also decides programmatic dependent launch: on where one trajectory's tiles fit one round of the resident warps, so that all
+// force warps finish together (pdl_mode).
+static int build_tiles(mdqt_handle* h) {
+  if (h->ilist) { cudaFree(h->ilist); h->ilist = nullptr; h->icount = 0; }
+  if (!h->items) return MDQT_OK;
+  std::vector<unsigned> list;
+  const int r0 = h->row0 / kTileIons, r1 = (h->row0 + h->nrows - 1) / kTileIons;  // the blocks of the handle's rows
+  for (int b = 0; b < h->B; b++) {
+    const int nbk = ((h->nb_host.empty() ? h->N : h->nb_host[b]) + kTileIons - 1) / kTileIons;
+    for (int I = 0; I < nbk; I++)
+      for (int J = I; J < nbk; J++)
+        if ((I >= r0 && I <= r1) || (J >= r0 && J <= r1)) list.push_back((unsigned)b << 16 | (unsigned)I << 8 | (unsigned)J);
+  }
+  if (pdl_mode() < 0) h->pdl = (h->B == 1 && h->nrows == h->N && list.size() <= 148u * kTileWarps) ? 1 : 0;
+  CU(cudaMalloc((void**)&h->ilist, sizeof(unsigned) * std::max<size_t>(list.size(), 1)));
+  CU(cudaMemcpy(h->ilist, list.data(), sizeof(unsigned) * list.size(), cudaMemcpyHostToDevice));
+  h->icount = (int)list.size();
+  return MDQT_OK;
+}
 
 static void plan_force(mdqt_handle* h) {
   // developer knobs (kernel A/B runs) are honoured on whole-system handles only: the ranks of a row-decomposed run must take the
@@ -150,15 +154,14 @@ static void plan_force(mdqt_handle* h) {
     const bool off = e && e[0] == '0' && h->p.plan_n == 0;
     // the chunk length must cover every trajectory's ions in <= 64 chunks even when n_ions exceeds the nominal plan_n
     const long long total_items = (long long)h->B * ((h->nrows + 31) / 32) * ((h->N + 7) / 8);  // bound for any chunk length
-    if (np <= kItemsMaxN && h->N <= 2 * np && total_items < (1LL << 24) && !off) {
+    if (np <= kItemsMaxN && h->N <= 2 * np && total_items < (1LL << 24) && h->B <= 65536 && !off) {
+      // pair-once tiles of 64-ion blocks (k_pairs_items): one partial per partner block, so the chain of additions a force term
+      // meets is at most jlen = 64 inside its tile plus nsplit partials; the diagnostic modes gather over chunks of the same length
       h->items = 1;
-      h->jlen = plan_items_jlen(np);
-      h->nsplit = (h->N + h->jlen - 1) / h->jlen;
+      h->jlen = kTileIons;
+      h->nsplit = (h->N + kTileIons - 1) / kTileIons;
       h->ipt = 1; h->jsub = 1; h->rg = 32;
       h->itiles = (h->nrows + 31) / 32;
-      // one trajectory whose items fit ONE round of the resident warps: all force warps finish together, which is when programmatic
-      // dependent launch pays (pdl_mode)
-      if (pdl_mode() < 0) h->pdl = (h->B == 1 && h->nrows == h->N && (long long)h->itiles * h->nsplit <= 148LL * 2 * 8) ? 1 : 0;
       return;
     }
   }
@@ -309,6 +312,10 @@ int mdqt_create(const mdqt_params* p, mdqt_handle** out) {
     mdqt_destroy(h);
     return fail(e == cudaErrorMemoryAllocation ? MDQT_ENOMEM : MDQT_ECUDA, m);
   }
+  if (int rc = build_tiles(h)) {
+    mdqt_destroy(h);
+    return rc;
+  }
   *out = h;
   return MDQT_OK;
 }
@@ -324,7 +331,6 @@ int mdqt_destroy(mdqt_handle* h) {
   if (h->tagged) cudaFree(h->tagged);
   if (h->clock) cudaFree(h->clock);
   if (h->nb) cudaFree(h->nb);
-  if (h->jl) cudaFree(h->jl);
   if (h->ilist) cudaFree(h->ilist);
   if (h->tags) cudaFree(h->tags);
   if (h->moments) cudaFree(h->moments);
@@ -448,53 +454,8 @@ int mdqt_set_ion_counts(mdqt_handle* h, const int32_t* n_ions) {
     CU(cudaMemcpy(h->nb, n_ions, sizeof(int) * (size_t)h->B, cudaMemcpyHostToDevice));
     h->nb_host.assign(n_ions, n_ions + h->B);
   }
-  // The chunk length of the item force kernel is a function of each trajectory's OWN ion count (plan_n == 0; a non-zero plan_n fixes one
-  // length for all): a job sums its forces in the same order alone (n_ions = its N) and in any batch, and every job gets the plan
-  // that fits its N (a nominal plan spills into a second round of items for the third of the jobs above N0 + 0.5 sigma).
-  {
-    const int old_nsplit = h->nsplit;
-    if (h->jl) { cudaFree(h->jl); h->jl = nullptr; }
-    plan_force(h);  // the uniform plan for N = n_ions (or plan_n)
-    if (n_ions && h->p.plan_n == 0) {
-      std::vector<int> jl(h->B);
-      int jmax = 8, nsmax = 1;
-      for (int b = 0; b < h->B; b++) {
-        jl[b] = plan_items_jlen(n_ions[b]);
-        jmax = std::max(jmax, jl[b]);
-        nsmax = std::max(nsmax, (n_ions[b] + jl[b] - 1) / jl[b]);
-      }
-      CU(cudaMalloc((void**)&h->jl, sizeof(int) * (size_t)h->B));
-      CU(cudaMemcpy(h->jl, jl.data(), sizeof(int) * (size_t)h->B, cudaMemcpyHostToDevice));
-      h->jlen = jmax; h->nsplit = nsmax;  // tile capacity and chunk-slot capacity of the batch
-      if (pdl_mode() < 0) h->pdl = (h->B == 1 && (long long)((n_ions[0] + 31) / 32) * h->nsplit <= 148LL * 2 * 8) ? 1 : 0;
-    }
-    // unequal ion counts leave ~8 % of the (trajectory, row group, chunk) slots empty, and a static walk over slots then gives the warps
-    // 29-34 real items each: hand the kernel the packed list of the non-empty items (two rows per lane: the batch instantiations)
-    if (h->ilist) { cudaFree(h->ilist); h->ilist = nullptr; h->icount = 0; }
-    if (n_ions && h->items && h->B > 1 && h->B < (1 << 14) && h->nsplit <= 1024 && h->N <= 64 * 256) {
-      std::vector<unsigned> list;
-      list.reserve((size_t)h->B * ((h->N + 63) / 64) * h->nsplit);
-      for (int b = 0; b < h->B; b++) {
-        const int jlb = (h->p.plan_n == 0) ? plan_items_jlen(n_ions[b]) : h->jlen;
-        const int groups = (n_ions[b] + 63) / 64, nch = (n_ions[b] + jlb - 1) / jlb;
-        for (int g = 0; g < groups; g++)
-          for (int ch = 0; ch < nch; ch++) list.push_back((unsigned)b << 18 | (unsigned)g << 10 | (unsigned)ch);
-      }
-      CU(cudaMalloc((void**)&h->ilist, sizeof(unsigned) * list.size()));
-      CU(cudaMemcpy(h->ilist, list.data(), sizeof(unsigned) * list.size(), cudaMemcpyHostToDevice));
-      h->icount = (int)list.size();
-    }
-    if (h->nsplit != old_nsplit) {  // the partial-sum buffers are sized by the number of chunk slots
-      cudaFree(h->Fpart); cudaFree(h->epot_partials);
-      h->Fpart = h->epot_partials = nullptr;
-      const size_t n1 = std::max<size_t>(h->nsplit > 1 ? (size_t)h->nsplit * state_elems(h) : 1, 1);
-      const size_t n2 = std::max<size_t>((size_t)h->itiles * h->nsplit * h->B, 1);
-      CU(cudaMalloc((void**)&h->Fpart, n1 * sizeof(double)));
-      CU(cudaMalloc((void**)&h->epot_partials, n2 * sizeof(double)));
-      CU(cudaMemset(h->Fpart, 0, n1 * sizeof(double)));
-      CU(cudaMemset(h->epot_partials, 0, n2 * sizeof(double)));
-    }
-  }
+  // the force tiles of every trajectory follow its OWN ion count: a job sums its forces in the same order alone and in any batch
+  if (int rc = build_tiles(h)) return rc;
   for (GraphEntry& g : h->graphs) cudaGraphExecDestroy(g.exec);  // captured arguments carried the old pointer
   h->graphs.clear();
   return MDQT_OK;
@@ -527,7 +488,7 @@ extern "C++" ForceArgs mdqt_force_args(mdqt_handle* h) {
   a.R = h->R; a.F = h->F; a.Fpart = h->Fpart; a.counters = h->counters;
   a.N = h->N; a.ld = h->ld; a.B = h->B; a.row0 = h->row0; a.nrows = h->nrows;
   a.nsplit = h->nsplit; a.jlen = h->jlen; a.ipt = h->ipt; a.jsub = h->jsub; a.rg = h->rg; a.Rfix = h->Rfix;
-  a.items = h->items; a.gcap = (h->nrows + 31) / 32; a.nb = h->nb; a.jl = h->jl; a.pdl = h->pdl; a.ilist = h->ilist; a.icount = h->icount;
+  a.items = h->items; a.gcap = (h->nrows + 31) / 32; a.nb = h->nb; a.pdl = h->pdl; a.ilist = h->ilist; a.icount = h->icount;
   a.mg_chunk = ((1ULL << 40) + h->nsplit - 1) / h->nsplit; a.mg_gcap = ((1ULL << 40) + a.gcap - 1) / a.gcap;
   { const int g2 = (h->nrows + 63) / 64; a.mg_gcap2 = ((1ULL << 40) + g2 - 1) / g2; }
   a.L = h->p.L; a.halfL = h->p.L / 2.; a.invL = 1.0 / h->p.L; a.kappa = h->p.kappa; a.rc2 = h->p.rcut * h->p.rcut;
@@ -584,7 +545,7 @@ static cudaEvent_t next_event(mdqt_handle* h) {
 extern "C++" int mdqt_enqueue_substeps(mdqt_handle* h, int nsub, int do_step, int do_kick, bool forces_partial) {
   if (h->forced_u && h->forced_cursor + nsub > h->forced_nsub) return fail(MDQT_ESTATE, "forced uniforms exhausted");
   QTArgs a = qt_args(h, nsub, do_step, do_kick);
-  if (forces_partial && forces_are_partial(force_args(h))) { a.fpart = h->Fpart; a.Fw = h->F; a.fp_jlen = h->jlen; a.jl = h->jl; }
+  if (forces_partial && forces_are_partial(force_args(h))) { a.fpart = h->Fpart; a.Fw = h->F; a.fp_jlen = h->jlen; }
   launch_substeps(a, h->qc, h->S, h->stream);
   if (h->forced_u) h->forced_cursor += nsub;
   h->substep += (uint64_t)nsub;
@@ -644,7 +605,7 @@ static int md_steps_graph(mdqt_handle* h, int nsteps) {
   fa.clock = h->clock; fa.clock_dtq = h->p.dtq; fa.clock_advance = 0;
   QTArgs qa = qt_args(h, ratio, 1, 1);
   qa.clock = h->clock; qa.t0 = 0.0; qa.substep0 = 0;
-  if (forces_are_partial(fa)) { qa.fpart = h->Fpart; qa.Fw = h->F; qa.fp_jlen = h->jlen; qa.jl = h->jl; }
+  if (forces_are_partial(fa)) { qa.fpart = h->Fpart; qa.Fw = h->F; qa.fp_jlen = h->jlen; }
   const bool stamp = h->timing == 2;
   if (stamp) {
     const size_t need = (size_t)nsteps * 2;

@@ -38,8 +38,7 @@ struct mdqt_handle {
   int pdl;  // programmatic dependent launch between the force and substep kernels (plan_force)
   int* nb;              // [B] per-trajectory ion counts on the device (ensembles with unequal N) or null
   std::vector<int> nb_host;
-  unsigned* ilist; int icount;  // compact item list of an unequal-N batch (ForceArgs.ilist) or null
-  int* jl;              // [B] per-trajectory chunk length of the item force kernel (set with nb when plan_n == 0) or null
+  unsigned* ilist; int icount;  // tile list of the pair-once force kernel (ForceArgs.ilist, build_tiles) or null
   uint64_t* seeds;      // [B] per-trajectory Philox keys or null
   int timing;  // 0 off; 1 = CUDA-event pair around every stream launch; 2 = %globaltimer stamps inside the replayed graph
   unsigned long long* stamps; size_t stamps_cap;  // [launch]{min start, max end} ns

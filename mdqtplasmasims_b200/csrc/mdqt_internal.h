@@ -10,6 +10,9 @@ constexpr int kExpTable = 1024;      // entries of the 2^(j/T) table used by the
 constexpr int kVelBins = 2001;       // KDE bins of output() (SU:120-123)
 constexpr int kTagBins = 4001;        // velocity bins of the tagged-ion distribution (MC408L:1069, FZ408L:835)
 constexpr int kMomentsPerRecord = 23; // 3 axis sums of v^2 + 4 tag sets x {count, sum v_x^1..4}
+// pair-once force tiles at small and medium N (k_pairs_items, mdqt_force.cu): ions per block, and resident warps per SM (one CTA)
+constexpr int kTileIons = 64;
+constexpr int kTileWarps = 12;
 
 struct ForceArgs {
   const double* R;   // [B][3][ld] all positions
@@ -36,15 +39,14 @@ struct ForceArgs {
   int half_l;        // rcut == L/2 exactly (every reference program): the cut-off is a power of two in fixed-point units
   double L, halfL, invL, invL_lo, kappa, rc2;  // 1/L = invL + invL_lo (double-double)
   double inv_u, rc2_u;  // fixed-point unit u = L/2^64: 1/u, and the squared cut-off in units u^2
-  // item-walking kernel (small and medium systems, any batch size): every warp of a persistent grid walks a static list of
-  // (trajectory, 32-row group, j chunk) items. items = 1 selects it; gcap = row groups per trajectory (at capacity)
+  // k_pairs_items (small and medium systems, any batch size): the persistent grid of the pair-once force tiles and of the diagnostics'
+  // gather over (trajectory, 32-row group, j chunk) items. items = 1 selects it; gcap = row groups per trajectory (at capacity)
   int items, gcap;
-  const int* jl;                          // item kernel: [B] chunk length of every trajectory, or null (all jlen); jlen = the largest
+  const int* jl;                          // gather: [B] chunk length of every trajectory, or null (all jlen, which plan_force sets)
   int pdl;                                // launch with programmatic stream serialisation (pdl_mode)
   unsigned long long mg_chunk, mg_gcap, mg_gcap2;  // ceil(2^40 / nsplit), ceil(2^40 / groups of 32 rows), ... of 64 rows: item index -> (b, g, chunk) without division
   const int* nb;     // [B] ions per trajectory (ensembles whose jobs drew different N, SU:299-337) or null: all N
-  // batches with unequal ion counts: the NON-EMPTY items at two rows per lane, packed b << 18 | 64-row group << 10 | chunk in slot
-  // order, so that the warps walk equal numbers of real items (the slot walk leaves them 29-34 each when 8 % of the slots are empty)
+  // the force tiles (b, I, J) the handle runs, packed b << 16 | I << 8 | J (mdqt_capi.cu, build_tiles)
   const unsigned* ilist; int icount;
   unsigned long long* stamp;  // {min start, max end} of this launch in %globaltimer ns (in-graph kernel timing) or null
 };
@@ -69,7 +71,7 @@ struct QTArgs {
   const int* nb;                          // [B] ions per trajectory or null (all N)
   const double* fpart; double* Fw;        // item-kernel partials [chunk][B][3][ld] to add up (then written to Fw), or null: F is complete
   int fp_jlen;                            // chunk length of those partials ...
-  const int* jl;                          // ... or [B], one per trajectory (per-trajectory ion counts)
+  const int* jl;                          // ... or [B], one per trajectory, or null (the force tiles: one length for all)
   const uint64_t* seeds;                  // [B] Philox key per trajectory or null (all `seed`)
   unsigned long long* stamp;              // {min start, max end} of this launch in %globaltimer ns, or null
   const double* clock;                    // {t, substep index (as uint64 bits)} in device memory: overrides t0/substep0 when non-null
